@@ -3,6 +3,9 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
     python bench.py --impl reference --steps K --warmup W    # the reference's algorithm on the host cores (oracle port)
+    python bench.py --steps K --warmup W --dump-outputs DIR  # also write what the timed steps computed, DIR/<name>.npy
+
+The sm_100a path loads the libacez.so that `python -m acezero_b200.build` left in the tree and writes nothing there.
 
 One JSON line on stdout (rank 0). A "step" is one ACE training iteration over a 5120-patch batch (head forward, fused
 reprojection loss, backward, GradScaler + AdamW; reference ace_trainer.py:499-640); the DSAC* pose solve
@@ -418,14 +421,24 @@ def run_reference(args):
 # ----------------------------------------------------------------------------------------------------------------
 # this repo's arm
 # ----------------------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy (float32 or float64, 64 MB at most in all), so that two builds run with the
+    same arguments can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a.astype(np.float64 if a.dtype.kind in "iu" or a.dtype == np.float64 else np.float32)
+        total += a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    assert total <= 64 << 20, total
+
+
 def run_ours(args):
     import torch.distributed as dist
-    from acezero_b200 import build
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
-    if rank == 0:
-        build.build()
     torch.cuda.set_device(local)
     dev = torch.device("cuda", local)
     if world > 1:
@@ -462,7 +475,7 @@ def run_ours(args):
 
     def step():
         s = (it[0] % n_batches) * bg
-        loop.train_iteration(perm[s:s + bg])
+        assert loop.train_iteration(perm[s:s + bg]), "the schedule ended inside the benchmark"
         it[0] += 1
 
     for _ in range(max(args.warmup, 3) + 2):   # +2: the CUDA graph is captured on the third call
@@ -482,6 +495,9 @@ def run_ours(args):
     ms_per_step = ms_total / args.steps
     iters_per_s = world * 1000.0 / ms_per_step      # 5120-patch iterations per second, whole job
     loss_final = float(head.stats[0])
+    # what the last timed training step leaves its caller (the sections below train further on the same head): the fp32
+    # head parameters and this rank's [loss sum, inlier count, valid count, non-finite flag]
+    outputs = {"train_head_params": head.params.clone(), "train_stats": head.stats.clone()}
 
     # ---------------- strong scaling: the SAME global batch of 5120 split over the ranks (what train_ace.py semantics mean:
     # --batch_size is the global batch; ace_trainer.py:613 divides by it) ----------------
@@ -605,10 +621,11 @@ def run_ours(args):
     e0.record()
     d_steps = max(3, min(args.steps, 20))
     for _ in range(d_steps):
-        dsac.forward_rgb_batch(maps, 525.0, 320.0, 240.0, **kw)
+        d_poses, d_inliers = dsac.forward_rgb_batch(maps, 525.0, 320.0, 240.0, **kw)
     e1.record()
     barrier()
     dsac_ms = max_over_ranks(e0.elapsed_time(e1) / d_steps)
+    outputs.update(dsac_poses=d_poses, dsac_inliers=d_inliers)
     poses_per_s = world * n_img * 1000.0 / dsac_ms
     # end to end: host scene coordinates in, host poses out
     t0 = time.perf_counter()
@@ -643,6 +660,7 @@ def run_ours(args):
     e1.record()
     barrier()
     enc_ms = max_over_ranks(e0.elapsed_time(e1) / e_steps)
+    outputs["encoder_head_scene_coords"] = sc_enc.clone()
     e0.record()
     for i in range(e_steps):
         enc.forward_nhwc(img_dev[i % 4], out=f_enc)
@@ -685,6 +703,8 @@ def run_ours(args):
         if world > 1:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     # ---------------- the reference's PyTorch path on this same GPU (rank 0, N = 1 only; SURVEY 8(d)(iii)) ----------------
     torch_gpu = None
     if world == 1 and not args.no_torch_baseline:
@@ -770,7 +790,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-torch-baseline", action="store_true")
     ap.add_argument("--no-pipeline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed steps computed in their last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the sm_100a path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

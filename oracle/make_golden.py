@@ -181,9 +181,56 @@ def pretrained_encoder_golden():
     print("wrote", dst, os.path.getsize(dst), "bytes")
 
 
+def refine_golden():
+    """The reference's `refine_poses.PoseRefiner` (refine_poses.py:85-250) in its three modes on the 7-pose dataset and the
+    index batch of tests/test_refine_cpu.py: poses it returns for the batch and for the whole dataset, before and after one
+    optimiser step on a fixed objective. Its `roma` dependency is stubbed with acezero_b200.refine's Gram-Schmidt /
+    Procrustes, so those two functions are pinned by their own tests, not by this fixture."""
+    from acezero_b200 import refine
+    sys.path.insert(0, str(REF))
+    roma = types.ModuleType("roma")
+    roma.special_gramschmidt = refine.special_gramschmidt
+    roma.special_procrustes = refine.special_procrustes
+    sys.modules["roma"] = roma
+    import refine_poses  # noqa: E402  (the reference's file)
+    torch.set_num_threads(8)
+    g = torch.Generator().manual_seed(1)
+    poses = []
+    for _ in range(7):
+        T = torch.eye(4)
+        T[:3, :3] = refine.special_procrustes(torch.randn(3, 3, generator=g))
+        T[:3, 3] = torch.randn(3, generator=g)
+        poses.append(T)
+    ds = type("DS", (), {"poses": poses, "__len__": lambda self: len(self.poses),
+                         "get_focal_length": lambda self, i: 525.0})()
+    idx = torch.tensor([[3], [0], [6], [3]], dtype=torch.int32)
+    orig = torch.stack([poses[i].inverse() for i in idx.view(-1).tolist()])
+    out = {"meta_torch_version": np.array(torch.__version__), "dataset_poses": torch.stack(poses).numpy()}
+    for mode in ("none", "naive", "mlp"):
+        opts = types.SimpleNamespace(pose_refinement=mode, pose_refinement_lr=0.001, pose_refinement_weight=0.1,
+                                     refinement_ortho="gram-schmidt")
+        torch.manual_seed(5)
+        r = refine_poses.PoseRefiner(ds, torch.device("cpu"), opts)
+        r.create_pose_buffer()
+        cur = r.get_current_poses(orig, idx)
+        out[f"pose_{mode}_current"] = cur.detach().numpy().copy()
+        out[f"pose_{mode}_all"] = r.get_all_current_poses().detach().cpu().numpy().copy()
+        if mode != "none":
+            r.zero_grad(set_to_none=True)
+            (cur[:, :3] * torch.arange(12.).view(1, 3, 4)).sum().backward()
+            r.step()
+            out[f"pose_{mode}_all_after_step"] = r.get_all_current_poses().detach().cpu().numpy().copy()
+    dst = REPO / "tests" / "golden" / "refine_golden.npz"
+    np.savez_compressed(dst, **out)
+    print("wrote", dst, os.path.getsize(dst), "bytes")
+
+
 if __name__ == "__main__":
     if "--pretrained-encoder" in sys.argv:
         pretrained_encoder_golden()
+    elif "--refine" in sys.argv:
+        refine_golden()
     else:
         main()
         pretrained_encoder_golden()
+        refine_golden()

@@ -28,3 +28,17 @@ def test_reference_arm_other_ranks_exit_quietly():
     out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1", "--warmup", "0"],
                          capture_output=True, text=True, timeout=120, cwd=str(ROOT), env=env)
     assert out.returncode == 0 and not [l for l in out.stdout.splitlines() if l.startswith("{")]
+
+
+def test_dump_outputs_writes_float_arrays(tmp_path):
+    """`--dump-outputs DIR`: one DIR/<name>.npy per output, integer and half results widened to float64 / float32."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, str(ROOT))
+    import bench
+    src = {"idx": torch.arange(5, dtype=torch.int32), "h": torch.linspace(0, 1, 7).half(), "d": torch.ones(2, 3, dtype=torch.float64)}
+    bench.dump_outputs(str(tmp_path / "out"), src)
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").glob("*.npy")}
+    assert {k: v.dtype for k, v in got.items()} == {"idx": np.float64, "h": np.float32, "d": np.float64}
+    for k, t in src.items():
+        np.testing.assert_array_equal(got[k], t.double().numpy())
