@@ -92,11 +92,11 @@ _lib = None
 
 # every symbol include/acez.h declares (the CPU test checks the .so exports all of them)
 EXPORTS = [
-    "acez_version", "acez_last_error", "acez_device_check", "acez_gemm_f16", "acez_gemm2cta_f16", "acez_debug_gemm2_clocks", "acez_repro_loss_fwd_bwd",
+    "acez_version", "acez_last_error", "acez_device_check", "acez_gemm_f16", "acez_repro_loss_fwd_bwd",
     "acez_head_param_count", "acez_head_workspace_bytes", "acez_head_plan_create", "acez_head_plan_destroy",
     "acez_head_sync_weights", "acez_head_input_ptr", "acez_head_plan_fused_chain", "acez_debug_chain_clocks", "acez_head_forward", "acez_head_forward_train",
     "acez_head_backward", "acez_head_train_fwd_bwd",
-    "acez_adamw_dp_shard", "acez_adamw_dp_reduce", "acez_adamw_dp_apply", "acez_adamw_dp_step", "acez_head_w16_ptr", "acez_gather_rows", "acez_gather_rows_multi", "acez_buffer_fill", "acez_adamw_step", "acez_schedule_init", "acez_schedule_step", "acez_gather_rows_multi_sched", "acez_dsac_workspace_bytes", "acez_dsac_forward_rgb_batch",
+    "acez_adamw_dp_shard", "acez_adamw_dp_step", "acez_head_w16_ptr", "acez_gather_rows", "acez_gather_rows_multi", "acez_buffer_fill", "acez_adamw_step", "acez_schedule_init", "acez_schedule_step", "acez_gather_rows_multi_sched", "acez_dsac_workspace_bytes", "acez_dsac_forward_rgb_batch",
     "acez_encoder_workspace_bytes", "acez_encoder_plan_create", "acez_encoder_plan_destroy", "acez_encoder_out_hw",
     "acez_encoder_forward", "acez_pointcloud_metrics",
 ]
@@ -115,8 +115,6 @@ def load():
     lib.acez_version.restype = C.c_int
     vp, i, f = C.c_void_p, C.c_int, C.c_float
     lib.acez_gemm_f16.argtypes = [C.POINTER(GemmDesc), vp]
-    lib.acez_gemm2cta_f16.argtypes = [C.POINTER(GemmDesc), vp]
-    lib.acez_debug_gemm2_clocks.argtypes = [vp, C.c_size_t]
     lib.acez_repro_loss_fwd_bwd.argtypes = [C.POINTER(LossParams), i] + [vp] * 13
     lib.acez_head_param_count.argtypes = [C.POINTER(HeadConfig)]
     lib.acez_head_param_count.restype = C.c_size_t
@@ -130,8 +128,6 @@ def load():
     lib.acez_head_w16_ptr.restype = vp
     lib.acez_adamw_dp_shard.argtypes = [C.c_size_t, i]
     lib.acez_adamw_dp_shard.restype = C.c_size_t
-    lib.acez_adamw_dp_reduce.argtypes = [vp, vp, i, i, C.c_size_t, vp, vp]
-    lib.acez_adamw_dp_apply.argtypes = [vp, vp, vp, i, i, C.c_size_t, vp, vp, vp, vp, vp, vp, vp, vp, vp, i, i, vp]
     lib.acez_adamw_dp_step.argtypes = [vp, vp, vp, vp, vp, i, i, C.c_size_t, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i, i, vp]
     lib.acez_head_input_ptr.argtypes = [vp]
     lib.acez_head_input_ptr.restype = vp

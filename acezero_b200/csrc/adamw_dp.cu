@@ -1,24 +1,25 @@
-// Data-parallel optimiser step over NVLink peer memory: the gradient all-reduce, GradScaler check, AdamW and the broadcast of
-// the new fp16 weights as TWO kernels that read / write the other GPUs' buffers directly (symmetric-memory peer pointers),
-// instead of an NCCL all-reduce of the full 8.4 MB gradient followed by a replicated AdamW over all 2.1 M parameters
-// (reference: ace_schedule.py:106-113 on one GPU; SURVEY.md section 8e for the sharding).
+// Data-parallel optimiser step over NVLink peer memory (acez_adamw_dp_step): the gradient all-reduce, GradScaler check, AdamW and
+// the broadcast of the new fp16 weights by kernels that read / write the other GPUs' buffers directly (symmetric-memory peer
+// pointers), instead of an NCCL all-reduce of the full 8.4 MB gradient followed by a replicated AdamW over all 2.1 M parameters
+// (reference: ace_schedule.py:106-113 on one GPU; SURVEY.md section 8e for the sharding). Rank r owns the parameter shard
+// [r S, (r+1) S), S = ceil(n / G / 8) * 8, and every rank computes the sum of ITS shard exactly once, in rank order, so all GPUs
+// see bit-identical weights. The ranks synchronise through epoch signals inside the kernels (below), so one call is a plain
+// sequence of kernels on the caller's stream and is captured in the iteration's CUDA graph.
 //
-//   rank r owns the parameter shard [r S, (r+1) S), S = ceil(n / G / 8) * 8:
-//   kernel 1 (reduce)  g_sum[i] = sum_q grads_q[i] for i in the shard, peers read in rank order 0..G-1 (every rank computes the
-//                      sum of ITS shard exactly once, so all GPUs later see bit-identical weights); fp16-range / inf check of the
-//                      summed shard -> this rank's flag, stored into EVERY rank's flag array (remote 4-byte stores); the 4 spare
-//                      slots behind the gradient (GradScaler flag of the ranks' local backward passes, loss / inlier / valid
-//                      sums) are summed by every rank for itself
-//   -- cross-GPU barrier (torch symmetric-memory barrier kernel) --
-//   kernel 2 (apply)   found = any rank's shard flag | non-finite flag slot; unless found: unscale, AdamW on the shard's fp32
-//                      master weights / moments (local), new weights rounded to fp16 and stored into EVERY rank's fp16 shadow
-//                      (the operand the forward / dgrad GEMMs read), the biases (read in fp32) into every rank's parameter
-//                      buffer; GradScaler.update() on every rank (same inputs, same state)
-//   -- cross-GPU barrier --
+// The step is ONE kernel (adamw_dp_fused_kernel) when the shard's parameter groups fit the registers of one co-resident grid.
+// Otherwise it runs as two kernels:
+//   reduce  block 0 packs the 4 spare slots behind this rank's gradient (+inf marker of the local GradScaler flag, loss / inlier /
+//           valid sums) and signals "gradient complete"; every block waits for every rank's signal. g_sum[i] = sum_q grads_q[i]
+//           for i in the shard; fp16-range / inf check of the summed shard -> this rank's flag, stored into EVERY rank's flag
+//           array (remote 4-byte stores); the spare slots are summed by every rank for itself. The last block signals "shard
+//           reduced".
+//   apply   waits for every rank's "shard reduced": found = any rank's shard flag | non-finite flag slot; unless found: unscale,
+//           AdamW on the shard's fp32 master weights / moments (local), new weights rounded to fp16 and stored into EVERY rank's
+//           fp16 shadow (the operand the forward / dgrad GEMMs read), the biases (read in fp32) into every rank's parameter
+//           buffer; GradScaler.update() on every rank (same inputs, same state). The last block signals "weights written" and
+//           waits for everybody's.
 // Traffic per GPU and iteration: (G-1)/G * 8.4 MB of gradient reads + (G-1)/G * 4.2 MB of weight writes over NVLink, AdamW
 // state traffic 1/G of the single-GPU kernel. fp32 master weights are valid on their owner only (gathered when exported).
-#include <stdlib.h>
-
 #include "common.cuh"
 
 namespace acez {
@@ -27,9 +28,8 @@ static constexpr int kC = 512;
 static constexpr size_t kLayerStride = (size_t)kC * kC + kC;
 static constexpr int kMaxRanks = 8;
 
-// Cross-GPU synchronisation INSIDE the kernels (acez_adamw_dp_step; the two-call interface leaves the barriers to the caller):
-// every rank's flag array (symmetric memory, int[kDpFlagInts]) also carries three rows of epoch signals, written by the peers
-// with st.release.sys over NVLink and polled locally with ld.acquire.sys:
+// Cross-GPU synchronisation INSIDE the kernels: every rank's flag array (symmetric memory, int[kDpFlagInts]) also carries three
+// rows of epoch signals, written by the peers with st.release.sys over NVLink and polled locally with ld.acquire.sys:
 //   [kSigGrads + q]   rank q's gradient of this iteration is complete        (sent by block 0 of q's reduce kernel)
 //   [kSigReduced + q] rank q has reduced its shard, its verdict flag is out  (sent by the last block of q's reduce kernel)
 //   [kSigApplied + q] rank q has written its shard of the new weights        (sent by the last block of q's apply kernel, which
@@ -104,26 +104,24 @@ __global__ void __launch_bounds__(256)
 adamw_dp_reduce_kernel(const DpPeers P, int world, int rank, size_t n, size_t shard, float* __restrict__ reduced,
                        float* __restrict__ my_grads /* nullable: this rank's gradient buffer (the spare slots are packed here) */,
                        const int* __restrict__ local_found_inf, const float* __restrict__ local_stats,
-                       unsigned int* __restrict__ sync_state /* nullable: [0] epoch, [1] block counter */) {
+                       unsigned int* __restrict__ sync_state /* [0] epoch, [1] block counter */) {
   pdl_wait();
-  const int epoch = sync_state != nullptr ? (int)sync_state[0] + 1 : 0;
-  if (sync_state != nullptr) {
-    // this rank's gradient is complete (stream order / the wait above): pack the spare slots behind it (the +inf marker of the
-    // local GradScaler flag, the loss / inlier / valid sums of the local backward pass), tell everybody, wait for everybody's
-    if (blockIdx.x == 0 && threadIdx.x == 0 && my_grads != nullptr) {
-      my_grads[n] = (*local_found_inf != 0) ? __int_as_float(0x7f800000) : 0.f;
-      my_grads[n + 1] = local_stats[0]; my_grads[n + 2] = local_stats[1]; my_grads[n + 3] = local_stats[2];
-    }
-    if (blockIdx.x == 0) {
-      __syncthreads();
-      if (threadIdx.x < world) {
-        __threadfence_system();
-        st_release_sys(P.flags[threadIdx.x] + kSigGrads + rank, epoch);
-      }
-    }
-    if (threadIdx.x < world) dp_wait_row(P.flags[rank], kSigGrads, threadIdx.x, epoch);
-    __syncthreads();
+  const int epoch = (int)sync_state[0] + 1;
+  // this rank's gradient is complete (stream order / the wait above): pack the spare slots behind it (the +inf marker of the
+  // local GradScaler flag, the loss / inlier / valid sums of the local backward pass), tell everybody, wait for everybody's
+  if (blockIdx.x == 0 && threadIdx.x == 0 && my_grads != nullptr) {
+    my_grads[n] = (*local_found_inf != 0) ? __int_as_float(0x7f800000) : 0.f;
+    my_grads[n + 1] = local_stats[0]; my_grads[n + 2] = local_stats[1]; my_grads[n + 3] = local_stats[2];
   }
+  if (blockIdx.x == 0) {
+    __syncthreads();
+    if (threadIdx.x < world) {
+      __threadfence_system();
+      st_release_sys(P.flags[threadIdx.x] + kSigGrads + rank, epoch);
+    }
+  }
+  if (threadIdx.x < world) dp_wait_row(P.flags[rank], kSigGrads, threadIdx.x, epoch);
+  __syncthreads();
   const size_t lo = (size_t)rank * shard;
   const size_t hi = lo + shard < n ? lo + shard : n;
   bool bad = false;
@@ -168,7 +166,7 @@ adamw_dp_reduce_kernel(const DpPeers P, int world, int rank, size_t n, size_t sh
   if (__syncthreads_or(bad ? 1 : 0) && threadIdx.x == 0) {
     for (int r = 0; r < world; ++r) *reinterpret_cast<volatile int*>(P.flags[r] + rank) = 1;   // remote stores: every rank learns this shard's verdict
   }
-  if (sync_state != nullptr && threadIdx.x == 0) {
+  if (threadIdx.x == 0) {
     __threadfence_system();   // this block's verdict stores before its arrival
     if (atomicAdd(sync_state + 1, 1u) == gridDim.x - 1) {
       sync_state[1] = 0u;
@@ -182,14 +180,12 @@ __global__ void adamw_dp_apply_kernel(const DpPeers P, int world, int rank, size
                                       float* __restrict__ p, float* __restrict__ m, float* __restrict__ v,
                                       const float* __restrict__ hyper, float* __restrict__ scaler_state, int* __restrict__ my_flags,
                                       int* __restrict__ found_inf_out, float* __restrict__ local_extras, int L, int C3,
-                                      unsigned int* __restrict__ sync_state /* nullable: [0] epoch */) {
+                                      unsigned int* __restrict__ sync_state /* [0] epoch */) {
   pdl_wait();
-  const int epoch = sync_state != nullptr ? (int)sync_state[0] + 1 : 0;
-  if (sync_state != nullptr) {
-    // every rank has reduced its shard: all verdict flags are final, and nobody computes with the old weights any more
-    if (threadIdx.x < world) dp_wait_row(my_flags, kSigReduced, threadIdx.x, epoch);
-    __syncthreads();
-  }
+  const int epoch = (int)sync_state[0] + 1;
+  // every rank has reduced its shard: all verdict flags are final, and nobody computes with the old weights any more
+  if (threadIdx.x < world) dp_wait_row(my_flags, kSigReduced, threadIdx.x, epoch);
+  __syncthreads();
   int found = 0;
   for (int r = 0; r < world; ++r) found |= my_flags[r];
   const float flag_slot = reduced[shard];    // sum of the ranks' +inf markers (local backward overflow)
@@ -281,8 +277,7 @@ __global__ void adamw_dp_apply_kernel(const DpPeers P, int world, int rank, size
   }
   __syncthreads();
   if (threadIdx.x == 0) {
-    if (sync_state != nullptr) __threadfence_system();   // this block's remote weight stores before its arrival
-    else __threadfence();
+    __threadfence_system();   // this block's remote weight stores before its arrival
     unsigned int* cnt = reinterpret_cast<unsigned int*>(scaler_state + 3);
     if (atomicAdd(cnt, 1u) == gridDim.x - 1) {
       if (found) { scaler_state[0] *= 0.5f; scaler_state[1] = 0.f; }
@@ -294,14 +289,12 @@ __global__ void adamw_dp_apply_kernel(const DpPeers P, int world, int rank, size
       *found_inf_out = found;
       for (int r = 0; r < world; ++r) my_flags[r] = 0;   // every block has read them (this is the last block to get here)
       *cnt = 0u;
-      if (sync_state != nullptr) {
-        sync_state[0] = (unsigned int)epoch;
-        __threadfence_system();
-        for (int r = 0; r < world; ++r) st_release_sys(P.flags[r] + kSigApplied + rank, epoch);
-        // the kernel completes only when every rank's shard of the new weights has landed in THIS rank's buffers: whatever
-        // follows in stream order (the next iteration's forward) may read them
-        for (int r = 0; r < world; ++r) dp_wait_row(my_flags, kSigApplied, r, epoch);
-      }
+      sync_state[0] = (unsigned int)epoch;
+      __threadfence_system();
+      for (int r = 0; r < world; ++r) st_release_sys(P.flags[r] + kSigApplied + rank, epoch);
+      // the kernel completes only when every rank's shard of the new weights has landed in THIS rank's buffers: whatever
+      // follows in stream order (the next iteration's forward) may read them
+      for (int r = 0; r < world; ++r) dp_wait_row(my_flags, kSigApplied, r, epoch);
     }
   }
 }
@@ -588,53 +581,6 @@ extern "C" size_t acez_adamw_dp_shard(size_t n, int world) {
   return (per + 7) / 8 * 8;
 }
 
-extern "C" int acez_adamw_dp_reduce(const void* const* peer_grads, void* const* peer_flags, int world, int rank, size_t n,
-                                    float* reduced_shard, acez_stream_t stream) {
-  ACEZ_REQUIRE(peer_grads && peer_flags && reduced_shard && world >= 1 && world <= kMaxRanks && rank >= 0 && rank < world,
-               "adamw_dp_reduce: bad arguments");
-  int rc = acez_device_check();
-  if (rc) return rc;
-  DpPeers P{};
-  for (int r = 0; r < world; ++r) {
-    ACEZ_REQUIRE(peer_grads[r] && peer_flags[r], "adamw_dp_reduce: null peer pointer %d", r);
-    P.grads[r] = reinterpret_cast<const float*>(peer_grads[r]);
-    P.flags[r] = reinterpret_cast<int*>(peer_flags[r]);
-  }
-  const size_t shard = acez_adamw_dp_shard(n, world);
-  const int grid = 2 * sm_count();
-  adamw_dp_reduce_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(P, world, rank, n, shard, reduced_shard, nullptr, nullptr, nullptr, nullptr);
-  ACEZ_CUDA(cudaGetLastError());
-  return ACEZ_OK;
-}
-
-extern "C" int acez_adamw_dp_apply(void* const* peer_w16, void* const* peer_w3h, void* const* peer_params, int world, int rank, size_t n,
-                                   const float* reduced_shard, float* params, float* exp_avg, float* exp_avg_sq,
-                                   const float* hyper_dev, float* scaler_state_dev, int* my_flags, int* found_inf_dev,
-                                   float* local_extras, int L, int C3, acez_stream_t stream) {
-  ACEZ_REQUIRE(peer_w16 && peer_w3h && peer_params && reduced_shard && params && exp_avg && exp_avg_sq && hyper_dev && scaler_state_dev &&
-                   my_flags && found_inf_dev && local_extras,
-               "adamw_dp_apply: null argument");
-  ACEZ_REQUIRE(world >= 1 && world <= kMaxRanks && rank >= 0 && rank < world && L >= 1 && (C3 == 3 || C3 == 4),
-               "adamw_dp_apply: bad arguments");
-  ACEZ_REQUIRE(n == (size_t)L * kLayerStride + (size_t)C3 * kC + (size_t)C3, "adamw_dp_apply: parameter count does not match the head");
-  int rc = acez_device_check();
-  if (rc) return rc;
-  DpPeers P{};
-  for (int r = 0; r < world; ++r) {
-    ACEZ_REQUIRE(peer_w16[r] && peer_w3h[r] && peer_params[r], "adamw_dp_apply: null peer pointer %d", r);
-    P.w16[r] = reinterpret_cast<__half*>(peer_w16[r]);
-    P.w3h[r] = reinterpret_cast<__half*>(peer_w3h[r]);
-    P.params[r] = reinterpret_cast<float*>(peer_params[r]);
-  }
-  const size_t shard = acez_adamw_dp_shard(n, world);
-  const int grid = 2 * sm_count();
-  adamw_dp_apply_kernel<<<grid, 256, 0, reinterpret_cast<cudaStream_t>(stream)>>>(P, world, rank, n, shard, reduced_shard, params, exp_avg,
-                                                                                  exp_avg_sq, hyper_dev, scaler_state_dev, my_flags,
-                                                                                  found_inf_dev, local_extras, L, C3, nullptr);
-  ACEZ_CUDA(cudaGetLastError());
-  return ACEZ_OK;
-}
-
 extern "C" int acez_adamw_dp_step(const void* const* peer_grads, void* const* peer_flags, void* const* peer_w16, void* const* peer_w3h,
                                   void* const* peer_params, int world, int rank, size_t n, float* reduced_shard, float* params,
                                   float* exp_avg, float* exp_avg_sq, const float* hyper_dev, float* scaler_state_dev,
@@ -668,16 +614,13 @@ extern "C" int acez_adamw_dp_step(const void* const* peer_grads, void* const* pe
   if (local_stats_dev != nullptr) {
     // the one-kernel step (the shard's parameter groups fit the registers of one co-resident grid); scratch = the four floats
     // behind the reduced-shard buffer
-    static const bool want_fused = [] { const char* e = getenv("ACEZ_DP_FUSED"); return e == nullptr || atoi(e) != 0; }();
     bool launched = false;
-    if (want_fused) {
-      float* my_grads = local_extras - n;
-      if (world <= 2) rc = launch_fused<2, 2>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
-      else if (world <= 4) rc = launch_fused<1, 4>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
-      else rc = launch_fused<1, 8>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
-      if (rc) return rc;
-      if (launched) return ACEZ_OK;
-    }
+    float* my_grads = local_extras - n;
+    if (world <= 2) rc = launch_fused<2, 2>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
+    else if (world <= 4) rc = launch_fused<1, 4>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
+    else rc = launch_fused<1, 8>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
+    if (rc) return rc;
+    if (launched) return ACEZ_OK;
   }
   // (blocks that poll a signal wait for REMOTE progress only, and the signals are sent by block 0 / the last block to finish:
   // no block of these grids waits for another block of its own GPU, so residency is not a correctness condition)

@@ -1,5 +1,5 @@
-// tcgen05 GEMM with cta_group::2: the batched weight-gradient GEMM of the training step (default since round 2; DESIGN.md
-// section 3.9) and the acez_gemm2cta_f16 entry of the C ABI.
+// tcgen05 GEMM with cta_group::2: the batched weight-gradient GEMM of the training step with the fused layer chain (DESIGN.md
+// section 3.9).
 //
 //   D[z][M,N] (fp32) = A[z] * B[z]      fp16 operands, fp32 accumulation in TMEM, operand layouts as in gemm.cuh
 //
@@ -17,8 +17,6 @@
 //   - tcgen05.commit.cta_group::2 ... multicast::cluster : stage release / accumulator-ready to BOTH CTAs
 // PTX forms follow the vendored CUTLASS headers (cute/arch/copy_sm100_tma.hpp, mma_sm100_umma.hpp,
 // tmem_allocator_sm100.hpp, cutlass/arch/barrier.h).
-#include <stdlib.h>
-
 #include "gemm2cta.cuh"
 
 namespace acez {
@@ -395,27 +393,11 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   }
 }
 
-static int encode2(CUtensorMap* tm, const __half* base, int mn_major, int rows_mn, int K, int ld, int batch, long long zstride,
-                   int tile_mn) {
-  uint64_t dims[3];
-  uint64_t strides[2];
-  uint32_t box[3];
-  if (!mn_major) {
-    dims[0] = (uint64_t)K; dims[1] = (uint64_t)rows_mn; dims[2] = (uint64_t)batch;
-    box[0] = 64; box[1] = (uint32_t)tile_mn; box[2] = 1;
-  } else {
-    dims[0] = (uint64_t)rows_mn; dims[1] = (uint64_t)K; dims[2] = (uint64_t)batch;
-    box[0] = 64; box[1] = 64; box[2] = 1;
-  }
-  strides[0] = (uint64_t)ld * 2;
-  strides[1] = (uint64_t)(batch > 1 ? zstride : (long long)dims[1] * ld) * 2;
-  return make_tensor_map(tm, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, base, dims, strides, box, nullptr, CU_TENSOR_MAP_SWIZZLE_128B);
-}
-
-template <bool A_MN, bool B_MN, int BN, bool C4>
+// MN-major operands (the weight gradient's dZ and X), 256-column tiles per CTA pair
+template <bool C4>
 static int launch2(const CUtensorMap& tmA, const CUtensorMap& tmB, const Gemm2Args& a, int batch, cudaStream_t stream, bool pdl) {
-  auto kern = gemm2cta_kernel<A_MN, B_MN, BN, C4>;
-  constexpr int T2_SMEM = T2Cfg<BN>::kSmem;
+  auto kern = gemm2cta_kernel<true, true, kGemm2BN, C4>;
+  constexpr int T2_SMEM = T2Cfg<kGemm2BN>::kSmem;
   static bool configured = false;
   if (!configured) {
     ACEZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM));
@@ -441,95 +423,11 @@ static int launch2(const CUtensorMap& tmA, const CUtensorMap& tmB, const Gemm2Ar
 }
 
 int gemm2_launch(const Gemm2Launch& L, cudaStream_t s, bool pdl) {
-  ACEZ_REQUIRE(L.a_mn == L.b_mn, "gemm2cta: operands must both be K-major or both MN-major");
-  ACEZ_REQUIRE(L.bn == 128 || L.bn == 256, "gemm2cta: bn must be 128 or 256");
-  const bool c4 = L.args.split_k == 2;   // on-chip split-K 2: cluster of four (two pairs per tile)
-  ACEZ_REQUIRE(!c4 || (L.bn == 256 && L.args.k_blocks >= 2), "gemm2cta: split-K 2 is built for 256-column tiles");
-  if (L.bn == 128) {
-    if (L.a_mn) return launch2<true, true, 128, false>(L.tmA, L.tmB, L.args, L.batch, s, pdl);
-    return launch2<false, false, 128, false>(L.tmA, L.tmB, L.args, L.batch, s, pdl);
+  if (L.args.split_k == 2) {   // on-chip split-K 2: cluster of four (two pairs per tile)
+    ACEZ_REQUIRE(L.args.k_blocks >= 2, "gemm2cta: split-K 2 needs at least two k-blocks");
+    return launch2<true>(L.tmA, L.tmB, L.args, L.batch, s, pdl);
   }
-  if (c4) {
-    if (L.a_mn) return launch2<true, true, 256, true>(L.tmA, L.tmB, L.args, L.batch, s, pdl);
-    return launch2<false, false, 256, true>(L.tmA, L.tmB, L.args, L.batch, s, pdl);
-  }
-  if (L.a_mn) return launch2<true, true, 256, false>(L.tmA, L.tmB, L.args, L.batch, s, pdl);
-  return launch2<false, false, 256, false>(L.tmA, L.tmB, L.args, L.batch, s, pdl);
+  return launch2<false>(L.tmA, L.tmB, L.args, L.batch, s, pdl);
 }
 
 }  // namespace acez
-
-static long long* g_gemm2_dbg = nullptr;
-// profiling probe: copies the per-CTA cycle counters of the last acez_gemm2cta_f16 call with ACEZ_GEMM2_DBG=1 (8 slots per CTA)
-extern "C" int acez_debug_gemm2_clocks(long long* host_out, size_t n_ctas) {
-  if (g_gemm2_dbg == nullptr || host_out == nullptr || n_ctas > 4096) return ACEZ_ERR_INVALID;
-  ACEZ_CUDA(cudaDeviceSynchronize());
-  ACEZ_CUDA(cudaMemcpy(host_out, g_gemm2_dbg, n_ctas * 8 * sizeof(long long), cudaMemcpyDeviceToHost));
-  return ACEZ_OK;
-}
-
-// C ABI: experimental entry (same descriptor as acez_gemm_f16; epilogue must be ACEZ_EPI_F32, plain fp32 store)
-extern "C" int acez_gemm2cta_f16(const acez_gemm_desc* d, acez_stream_t stream) {
-  using namespace acez;
-  ACEZ_REQUIRE(d != nullptr, "gemm2cta: null desc");
-  int rc = acez_device_check();
-  if (rc) return rc;
-  ACEZ_REQUIRE(d->epilogue == ACEZ_EPI_F32 && d->out32 != nullptr && d->ldo32 % 4 == 0, "gemm2cta: fp32 output only");
-  ACEZ_REQUIRE(d->M > 0 && d->N > 0 && d->K > 0 && d->K % T2_BK == 0 && d->N % 32 == 0, "gemm2cta: bad shape");
-  ACEZ_REQUIRE(d->a_mn_major == d->b_mn_major, "gemm2cta: probe supports K-major x K-major and MN-major x MN-major");
-  Gemm2Launch L{};
-  L.batch = d->batch > 0 ? d->batch : 1;
-  L.bn = (d->bn == 128) ? 128 : 256;  // columns per pair
-  L.a_mn = d->a_mn_major; L.b_mn = d->b_mn_major;
-  rc = encode2(&L.tmA, reinterpret_cast<const __half*>(d->A), d->a_mn_major, d->M, d->K, d->lda, L.batch, d->a_zstride, T2_BM);
-  if (rc) return rc;
-  rc = encode2(&L.tmB, reinterpret_cast<const __half*>(d->B), d->b_mn_major, d->N, d->K, d->ldb, L.batch, d->b_zstride, L.bn / 2);
-  if (rc) return rc;
-  Gemm2Args& a = L.args;
-  a.M = d->M; a.N = d->N; a.k_blocks = d->K / T2_BK;
-  a.tiles_n = (d->N + L.bn - 1) / L.bn;
-  a.out32 = d->out32; a.out32_zstride = d->out32_zstride; a.ldo32 = d->ldo32;
-  a.bias_grad = d->bias_grad; a.bias_grad_zstride = d->bias_grad_zstride;
-  if (d->bias_grad != nullptr) {
-    // probe entry: the partial-sum workspace and its arrival counters live in a process-wide scratch allocation
-    static float* g_part = nullptr;
-    static unsigned int* g_count = nullptr;
-    static size_t g_cap = 0;
-    const int tiles_m = (d->M + 2 * T2_BM - 1) / (2 * T2_BM);
-    const size_t need = (size_t)L.batch * tiles_m * a.tiles_n * 2 * T2_BM;
-    if (need > g_cap) {
-      if (g_part) cudaFree(g_part);
-      ACEZ_CUDA(cudaMalloc(&g_part, need * sizeof(float)));
-      g_cap = need;
-    }
-    if (g_count == nullptr) {
-      ACEZ_CUDA(cudaMalloc(&g_count, 4096 * sizeof(unsigned int)));
-      ACEZ_CUDA(cudaMemset(g_count, 0, 4096 * sizeof(unsigned int)));
-    }
-    ACEZ_REQUIRE((size_t)L.batch * tiles_m <= 4096, "gemm2cta: too many row tiles for the probe's counters");
-    a.bias_part = g_part;
-    a.bias_count = g_count;
-  }
-  {
-    // probe entry: ACEZ_GEMM2_SPLITK=2 contracts each tile in two halves (two CTAs per tile and half)
-    static const int want_split = [] { const char* e = getenv("ACEZ_GEMM2_SPLITK"); return e != nullptr ? atoi(e) : 1; }();
-    a.split_k = (want_split == 2 && a.k_blocks >= 2 && L.bn == 256) ? 2 : 1;
-  }
-  {
-    static const bool want = [] { const char* e = getenv("ACEZ_GEMM2_DBG"); return e != nullptr && atoi(e) != 0; }();
-    static long long* g_dbg = nullptr;
-    if (want) {
-      if (g_dbg == nullptr) ACEZ_CUDA(cudaMalloc(&g_dbg, 8 * 4096 * sizeof(long long)));
-      ACEZ_CUDA(cudaMemsetAsync(g_dbg, 0, 8 * 4096 * sizeof(long long), reinterpret_cast<cudaStream_t>(stream)));
-      a.dbg = g_dbg;
-      g_gemm2_dbg = g_dbg;
-    }
-  }
-  if (d->a_lbo) a.a_lbo = d->a_lbo;
-  if (d->a_sbo) a.a_sbo = d->a_sbo;
-  if (d->a_kstep) a.a_kstep = d->a_kstep;
-  if (d->b_lbo) a.b_lbo = d->b_lbo;
-  if (d->b_sbo) a.b_sbo = d->b_sbo;
-  if (d->b_kstep) a.b_kstep = d->b_kstep;
-  return gemm2_launch(L, reinterpret_cast<cudaStream_t>(stream));
-}

@@ -1,4 +1,4 @@
-// EXPERIMENTAL cta_group::2 GEMM (gemm2cta.cu): launch descriptor shared with head.cu (opt-in weight-gradient path).
+// cta_group::2 GEMM (gemm2cta.cu): launch descriptor of the batched weight gradient that head.cu runs after the fused dgrad chain.
 #pragma once
 #include "gemm.cuh"
 
@@ -18,16 +18,16 @@ struct Gemm2Args {
   uint32_t a_lbo, a_sbo, a_kstep, b_lbo, b_sbo, b_kstep;
   int split_k;           // 1, or 2 (256-column tiles only): a cluster of four CTAs = two pairs per tile, each contracting half of the
                          // k-blocks; the second pair's accumulator travels to the first through distributed shared memory
-  long long* dbg;        // nullable (ACEZ_GEMM2_DBG=1): per CTA [0] MMA-warp cycles waiting for operands, [1] MMA loop cycles,
+  long long* dbg;        // nullable (no caller sets it): per CTA [0] MMA-warp cycles waiting for operands, [1] MMA loop cycles,
                          // [2] producer cycles waiting for free stages, [3] producer loop cycles, [4] epilogue cycles
 };
 
+static constexpr int kGemm2BN = 256;  // columns per CTA pair
+
 struct Gemm2Launch {
-  CUtensorMap tmA, tmB;  // A: box of this CTA's 128 rows; B: box of this CTA's bn / 2 rows (K-major) or 64 x 64 boxes (MN-major)
+  CUtensorMap tmA, tmB;  // MN-major operands [z][K][M] / [z][K][N], 64 x 64 boxes
   Gemm2Args args;
   int batch;
-  int bn;                // 128 or 256 columns per CTA pair
-  int a_mn, b_mn;        // 0 = K-major, 1 = MN-major (both equal)
 };
 
 // pdl: programmatic dependent launch (only when the stream predecessor is a kernel)

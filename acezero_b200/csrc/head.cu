@@ -55,18 +55,11 @@ struct acez_head_plan {
   int prepared_training;
   std::vector<acez::GemmLaunch> fwd;
   std::vector<acez::GemmLaunch> dgrad;
-  acez::GemmLaunch wgrad;                    // all layers in one launch (grid.z = layer)
-  std::vector<acez::GemmLaunch> wgrad_layer;  // one launch per layer, run on a side stream under the dgrad chain
+  acez::GemmLaunch wgrad;    // per-layer plans: all weight gradients in one cta_group::1 launch (grid.z = layer)
   // fused layer chains (head_chain.cu): one launch for all hidden layers of a pass
   int use_chain;
   acez::ChainLaunch chain_fwd, chain_bwd;
-  int use_wgrad2;              // ACEZ_WGRAD_2CTA=1 (experimental): batched weight gradient on cta_group::2 tiles (gemm2cta.cu)
-  acez::Gemm2Launch wgrad2;
-  cudaStream_t side_stream;
-  cudaEvent_t ev_dz[32];
-  cudaEvent_t ev_join;
-  bool side_ready;
-  int overlap_wgrad;
+  acez::Gemm2Launch wgrad2;  // chain plans: all weight gradients in one cta_group::2 launch (gemm2cta.cu)
 };
 
 namespace acez {
@@ -760,95 +753,60 @@ static int head_prepare(acez_head_plan* h, int rows, int training) {
       rc = gemm_finalize(&h->dgrad[l]);
       if (rc) return rc;
     }
-    // all weight gradients in one launch: grid.z = layer, no split-K, plain fp32 stores
-    GemmProblem p{};
-    p.A = h->DZ; p.B = h->ACT;
-    p.a_mn = 1; p.b_mn = 1;
-    p.M = kC; p.N = kC; p.K = (rows + 63) / 64 * 64; p.batch = L;
-    p.a_zstride = (long long)h->act_stride; p.b_zstride = (long long)h->act_stride;
-    p.lda = kC; p.ldb = kC;
-    {
-      const char* e = getenv("ACEZ_WGRAD_BN");
+    // all weight gradients in one launch: grid.z = layer, dZ and X MN-major, plain fp32 stores. Contraction rows beyond `rows`
+    // must read as zero: the operand maps carry the true row count so that TMA zero-fills
+    const uint64_t dims[3] = {(uint64_t)kC, (uint64_t)rows, (uint64_t)L};
+    const uint64_t strides[2] = {(uint64_t)kC * 2, (uint64_t)h->act_stride * 2};
+    const uint32_t box[3] = {64, 64, 1};
+    if (h->use_chain) {
+      // 256 x 256 tiles of CTA pairs with an on-chip split-K 2: a cluster of four = two pairs per tile, 128 CTAs; the tensor pipe
+      // runs at 87 % per CTA instead of the 50 % of 128-column tiles (round-2 cycle counters) and the second pair's accumulator
+      // travels through distributed shared memory. Measured (round 2, warm graph replays): 171.0 us per iteration against 180.6 us
+      // with 256 x 128 tiles and no split; the launch alone takes ~35 us against 44.7 us for the cta_group::1 kernel below
+      Gemm2Launch& W = h->wgrad2;
+      W = Gemm2Launch{};
+      int rc = make_tensor_map(&W.tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, h->DZ, dims, strides, box, nullptr,
+                               CU_TENSOR_MAP_SWIZZLE_128B);
+      if (rc) return rc;
+      rc = make_tensor_map(&W.tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, h->ACT, dims, strides, box, nullptr,
+                           CU_TENSOR_MAP_SWIZZLE_128B);
+      if (rc) return rc;
+      W.batch = L;
+      Gemm2Args& g = W.args;
+      g.M = kC; g.N = kC; g.k_blocks = (rows + 63) / 64;
+      g.tiles_n = kC / kGemm2BN;
+      g.out32 = h->grads; g.out32_zstride = (long long)kLayerStride; g.ldo32 = kC;
+      g.bias_grad = h->grads + (size_t)kC * kC; g.bias_grad_zstride = (long long)kLayerStride;
+      g.bias_part = h->WBIAS;
+      g.bias_count = h->BLKCOUNT + 8;   // [L][2] arrival counters behind the tail's; zeroed once with it (launch_tail)
+      g.split_k = g.k_blocks >= 2 ? 2 : 1;
+      g.a_lbo = 8192; g.a_sbo = 1024; g.a_kstep = 2048;
+      g.b_lbo = 8192; g.b_sbo = 1024; g.b_kstep = 2048;
+    } else {
       // measured (round 1, warm graph replays): 128 x 128 tiles / 128 CTAs: 220 us per iteration, 128 x 256 / 64 CTAs: 231 us
-      p.bn = (e != nullptr && atoi(e) == 256) ? 256 : 128;
-    }
-    p.epi = EPI_WGRAD;
-    int rc = gemm_prepare(&h->wgrad, p);
-    if (rc) return rc;
-    // contraction rows beyond `rows` must read as zero: rebuild the maps with the true row count so TMA zero-fills
-    {
-      uint64_t dims[3] = {(uint64_t)kC, (uint64_t)rows, (uint64_t)L};
-      uint64_t strides[2] = {(uint64_t)kC * 2, (uint64_t)h->act_stride * 2};
-      uint32_t box[3] = {64, 64, 1};
+      GemmProblem p{};
+      p.A = h->DZ; p.B = h->ACT;
+      p.a_mn = 1; p.b_mn = 1;
+      p.M = kC; p.N = kC; p.K = (rows + 63) / 64 * 64; p.batch = L;
+      p.a_zstride = (long long)h->act_stride; p.b_zstride = (long long)h->act_stride;
+      p.lda = kC; p.ldb = kC;
+      p.bn = 128;
+      p.epi = EPI_WGRAD;
+      int rc = gemm_prepare(&h->wgrad, p);
+      if (rc) return rc;
       rc = make_tensor_map(&h->wgrad.tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, h->DZ, dims, strides, box, nullptr,
                            CU_TENSOR_MAP_SWIZZLE_128B);
       if (rc) return rc;
       rc = make_tensor_map(&h->wgrad.tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, h->ACT, dims, strides, box, nullptr,
                            CU_TENSOR_MAP_SWIZZLE_128B);
       if (rc) return rc;
-    }
-    if (h->use_wgrad2) {
-      // the same operands (MN-major DZ / ACT, rows beyond `rows` zero-filled by TMA) on 256 x bn tiles of CTA pairs
-      Gemm2Launch& W = h->wgrad2;
-      W = Gemm2Launch{};
-      W.tmA = h->wgrad.tmA;
-      W.tmB = h->wgrad.tmB;
-      W.batch = L;
-      W.a_mn = W.b_mn = 1;
-      {
-        // 256 x 256 tiles with an on-chip split-K 2 (default): a cluster of four = two pairs per tile, 128 CTAs; the tensor pipe
-        // runs at 87 % per CTA instead of the 50 % of 128-column tiles (round-2 cycle counters) and the second pair's
-        // accumulator travels through distributed shared memory: 171.0 vs 180.6 us per iteration. ACEZ_WGRAD_2CTA_BN=128: 256 x
-        // 128 tiles per pair, 64 pairs, no split
-        const char* e = getenv("ACEZ_WGRAD_2CTA_BN");
-        W.bn = (e != nullptr && atoi(e) == 128) ? 128 : 256;
-      }
-      Gemm2Args& g = W.args;
-      g.M = kC; g.N = kC; g.k_blocks = (rows + 63) / 64;
-      g.tiles_n = kC / W.bn;
-      g.out32 = h->grads; g.out32_zstride = (long long)kLayerStride; g.ldo32 = kC;
-      g.bias_grad = h->grads + (size_t)kC * kC; g.bias_grad_zstride = (long long)kLayerStride;
-      g.bias_part = h->WBIAS;
-      g.bias_count = h->BLKCOUNT + 8;   // [L][2] arrival counters behind the tail's; zeroed once with it (launch_tail)
-      g.split_k = (W.bn == 256 && g.k_blocks >= 2) ? 2 : 1;   // on-chip split-K 2 (cluster of four)
-      g.a_lbo = 8192; g.a_sbo = 1024; g.a_kstep = 2048;
-      g.b_lbo = 8192; g.b_sbo = 1024; g.b_kstep = 2048;
-    }
-    GemmArgs& a = h->wgrad.args;
-    a.out32 = h->grads;
-    a.out32_zstride = (long long)kLayerStride;
-    a.ldo32 = kC;
-    a.bias_grad = h->grads + (size_t)kC * kC;
-    a.bias_grad_zstride = (long long)kLayerStride;
-    rc = gemm_finalize(&h->wgrad);
-    if (rc) return rc;
-    // per-layer variant (128 x 128 tiles, 16 CTAs per layer): small enough to run on the SMs the 80-CTA dgrad kernels
-    // leave idle, so the weight gradients are computed concurrently with the dgrad chain on a second stream
-    h->wgrad_layer.assign(L, GemmLaunch{});
-    for (int l = 0; l < L; ++l) {
-      GemmProblem q = p;
-      q.A = h->DZ + (size_t)l * h->act_stride;
-      q.B = h->ACT + (size_t)l * h->act_stride;
-      q.batch = 1;
-      q.bn = 128;
-      rc = gemm_prepare(&h->wgrad_layer[l], q);
-      if (rc) return rc;
-      uint64_t dims[3] = {(uint64_t)kC, (uint64_t)rows, 1};
-      uint64_t strides[2] = {(uint64_t)kC * 2, (uint64_t)h->act_stride * 2};
-      uint32_t box[3] = {64, 64, 1};
-      rc = make_tensor_map(&h->wgrad_layer[l].tmA, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, q.A, dims, strides, box, nullptr,
-                           CU_TENSOR_MAP_SWIZZLE_128B);
-      if (rc) return rc;
-      rc = make_tensor_map(&h->wgrad_layer[l].tmB, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, q.B, dims, strides, box, nullptr,
-                           CU_TENSOR_MAP_SWIZZLE_128B);
-      if (rc) return rc;
-      GemmArgs& b = h->wgrad_layer[l].args;
-      b.out32 = h->grads + (size_t)l * kLayerStride;
-      b.out32_zstride = 0;
-      b.ldo32 = kC;
-      b.bias_grad = h->grads + (size_t)l * kLayerStride + (size_t)kC * kC;
-      b.bias_grad_zstride = 0;
-      rc = gemm_finalize(&h->wgrad_layer[l]);
+      GemmArgs& a = h->wgrad.args;
+      a.out32 = h->grads;
+      a.out32_zstride = (long long)kLayerStride;
+      a.ldo32 = kC;
+      a.bias_grad = h->grads + (size_t)kC * kC;
+      a.bias_grad_zstride = (long long)kLayerStride;
+      rc = gemm_finalize(&h->wgrad);
       if (rc) return rc;
     }
   }
@@ -912,16 +870,6 @@ static void fill_tail_common(const acez_head_plan* h, int rows, TailArgs& t) {
 
 static int tail_grid(int rows) { return (rows + kTailRows - 1) / kTailRows; }
 
-static int ensure_side_stream(acez_head_plan* h) {
-  if (!h->side_ready) {
-    ACEZ_CUDA(cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < h->L; ++i) ACEZ_CUDA(cudaEventCreateWithFlags(&h->ev_dz[i], cudaEventDisableTiming));
-    ACEZ_CUDA(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-    h->side_ready = true;
-  }
-  return ACEZ_OK;
-}
-
 // tail (+ fc3 gradient) launch sequence shared by the training entries
 static int launch_tail(acez_head_plan* h, TailArgs& t, int rows, cudaStream_t s, int* nonfinite, bool with_fc3_grad,
                        bool pdl) {
@@ -952,57 +900,22 @@ static int launch_tail(acez_head_plan* h, TailArgs& t, int rows, cudaStream_t s,
   return ACEZ_OK;
 }
 
-// dgrad chain + weight gradients. Overlapped mode: layer l's wgrad is enqueued on the plan's side stream as soon as
-// DZ[l] exists (event after the kernel that produced it) and runs on the SMs the dgrad kernels leave idle; the main
-// stream joins at the end. Works eagerly and under stream capture (fork / join through events).
+// dgrad pass + weight gradients
 static int launch_backward_gemms(acez_head_plan* h, cudaStream_t s, int* nonfinite) {
-  const int L = h->L;
-  if (h->use_chain && L >= 2) {
+  if (h->use_chain) {
     h->chain_bwd.args.nonfinite = nonfinite;
     int rc = chain_launch(h->chain_bwd, s, /*pdl=*/true);  // predecessor: fc3_reduce_kernel
     if (rc) return rc;
-    if (h->use_wgrad2) {
-      h->wgrad2.args.nonfinite = nonfinite;
-      rc = gemm2_launch(h->wgrad2, s, /*pdl=*/true);
-    } else {
-      h->wgrad.args.nonfinite = nonfinite;
-      rc = gemm_launch(h->wgrad, s);
-    }
+    h->wgrad2.args.nonfinite = nonfinite;  // fp16-overflow / inf check of the weight gradients in the epilogue
+    return gemm2_launch(h->wgrad2, s, /*pdl=*/true);
+  }
+  for (int l = h->L - 1; l >= 1; --l) {
+    h->dgrad[l].args.nonfinite = nonfinite;
+    int rc = gemm_launch(h->dgrad[l], s);
     if (rc) return rc;
-    return ACEZ_OK;
   }
-  if (!h->overlap_wgrad) {
-    for (int l = L - 1; l >= 1; --l) {
-      h->dgrad[l].args.nonfinite = nonfinite;
-      int rc = gemm_launch(h->dgrad[l], s);
-      if (rc) return rc;
-    }
-    h->wgrad.args.nonfinite = nonfinite;  // fp16-overflow / inf check of the weight gradients in the epilogue
-    return gemm_launch(h->wgrad, s);
-  }
-  if (!h->side_ready) {
-    ACEZ_CUDA(cudaStreamCreateWithFlags(&h->side_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < L; ++i) ACEZ_CUDA(cudaEventCreateWithFlags(&h->ev_dz[i], cudaEventDisableTiming));
-    ACEZ_CUDA(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
-    h->side_ready = true;
-  }
-  cudaStream_t side = h->side_stream;
-  for (int l = L - 1; l >= 0; --l) {
-    // DZ[l] is complete here (tail for l = L-1, dgrad l+1 otherwise)
-    ACEZ_CUDA(cudaEventRecord(h->ev_dz[l], s));
-    ACEZ_CUDA(cudaStreamWaitEvent(side, h->ev_dz[l], 0));
-    h->wgrad_layer[l].args.nonfinite = nonfinite;
-    int rc = gemm_launch(h->wgrad_layer[l], side, /*pdl=*/false);
-    if (rc) return rc;
-    if (l >= 1) {
-      h->dgrad[l].args.nonfinite = nonfinite;
-      rc = gemm_launch(h->dgrad[l], s, /*pdl=*/false);  // an event record sits between consecutive dgrad kernels
-      if (rc) return rc;
-    }
-  }
-  ACEZ_CUDA(cudaEventRecord(h->ev_join, side));
-  ACEZ_CUDA(cudaStreamWaitEvent(s, h->ev_join, 0));
-  return ACEZ_OK;
+  h->wgrad.args.nonfinite = nonfinite;
+  return gemm_launch(h->wgrad, s);
 }
 
 }  // namespace acez
@@ -1073,25 +986,12 @@ extern "C" int acez_head_plan_create(const acez_head_config* cfg, float* params,
   h->BLKPART = reinterpret_cast<float*>(base + lo.blkpart);
   h->BLKCOUNT = reinterpret_cast<unsigned int*>(base + lo.blkpart + 4096 * 8 * sizeof(float));
   h->counters_zeroed = false;
-  h->side_ready = false;
-  {
-    const char* e = getenv("ACEZ_WGRAD_OVERLAP");
-    // measured on B200 (round 1): the 16-CTA per-layer kernels are bound by the per-SM L2 ingest rate (~20 us each)
-    // and become the critical path (393 us / iteration vs 216 us batched), so the batched launch stays the default
-    h->overlap_wgrad = (e == nullptr) ? 0 : atoi(e);
-  }
   {
     // Default: all hidden layers of the forward / dgrad pass in one cluster kernel each (head_chain.cu); measured on
     // B200 (round 1, b = 5120): 0.212 ms per training iteration against 0.232 ms with one GEMM launch per layer.
     // ACEZ_HEAD_CHAIN=0 selects the per-layer tcgen05 GEMM path (also used when the head is deeper than the chain holds).
     const char* e = getenv("ACEZ_HEAD_CHAIN");
     h->use_chain = ((e == nullptr || atoi(e) != 0) && h->L <= kChainMaxSteps) ? 1 : 0;
-  }
-  {
-    // batched weight gradient on cta_group::2 tiles (gemm2cta.cu, 256 x 128 per SM pair): validated in round 2, 35.4 vs 44.7 us
-    // for the 8 x 512 x 512 x 5120 launch; ACEZ_WGRAD_2CTA=0 selects the cta_group::1 kernel of gemm.cu
-    const char* e = getenv("ACEZ_WGRAD_2CTA");
-    h->use_wgrad2 = (e == nullptr || atoi(e) != 0) ? 1 : 0;
   }
   h->act_stride = (size_t)cfg->max_rows * kC;
   h->prepared_rows = -1;
@@ -1101,12 +1001,6 @@ extern "C" int acez_head_plan_create(const acez_head_config* cfg, float* params,
 }
 
 extern "C" void acez_head_plan_destroy(acez_head_plan* plan) {
-  if (plan == nullptr) return;
-  if (plan->side_ready) {
-    cudaStreamDestroy(plan->side_stream);
-    for (int i = 0; i < plan->L; ++i) cudaEventDestroy(plan->ev_dz[i]);
-    cudaEventDestroy(plan->ev_join);
-  }
   delete plan;
 }
 
@@ -1301,7 +1195,7 @@ extern "C" int acez_adamw_step(float* params, const float* grads, float* exp_avg
   cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
   const int grid = 8 * sm_count();
   if (use_scaler == 1 || use_scaler == 3) {  // 2 = the caller's flag already covers every gradient (acez_head_train_fwd_bwd does)
-    // 3 (data parallel, experimental): one more element behind the gradient is checked too - the slot in which the ranks'
+    // 3 (data parallel through NCCL): one more element behind the gradient is checked too - the slot in which the ranks'
     // local GradScaler flags travelled through the all-reduce (+inf when any rank overflowed)
     rc = launch_pdl(grad_check_kernel, dim3(grid), dim3(256), 0, s, false, grads, n + (use_scaler == 3 ? 1 : 0), found_inf_dev);
     if (rc) return rc;

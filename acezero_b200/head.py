@@ -258,8 +258,6 @@ class HeadEngine:
         self.dp_flags = sm.empty(64, dtype=torch.int32, device=self.device).zero_()
         self.dp_sync_state = torch.zeros(4, dtype=torch.int32, device=self.device)
         import os
-        # cross-GPU synchronisation inside the two optimiser kernels (default); 0: torch symmetric-memory barriers around them
-        self.dp_signals = os.environ.get("ACEZ_DP_SIGNALS", "1") != "0"
         torch.cuda.synchronize()
         hp = sm.rendezvous(self.params, g)
         hg = sm.rendezvous(self.grads_full, g)
@@ -283,7 +281,7 @@ class HeadEngine:
             mc = None
         self.dp_multicast = mc
         self.peer = {
-            "world": world, "rank": rank, "shard": shard, "handles": (hp, hg, hw, hf), "barrier": hg,
+            "world": world, "rank": rank, "shard": shard, "handles": (hp, hg, hw, hf),
             "params": arr(hp.buffer_ptrs), "grads": arr(hg.buffer_ptrs), "flags": arr(hf.buffer_ptrs),
             "w16": arr([p + off16 for p in hw.buffer_ptrs]), "w3h": arr([p + off3 for p in hw.buffer_ptrs]),
             "reduced": torch.zeros(shard + 4, device=self.device, dtype=torch.float32),
@@ -291,30 +289,17 @@ class HeadEngine:
         return self.peer
 
     def adamw_step_peers(self, stream=None):
-        """Optimiser step of one data-parallel iteration over peer memory (csrc/adamw_dp.cu): barrier, reduce this rank's shard
-        of the gradient from all ranks, barrier, AdamW on the shard + the new fp16 weights to all ranks, barrier."""
+        """Optimiser step of one data-parallel iteration over peer memory (csrc/adamw_dp.cu): reduce this rank's shard of the
+        gradient from all ranks, AdamW on the shard + the new fp16 weights to all ranks, synchronised across the GPUs inside
+        the kernels (no host-side barrier: the step can be captured in a CUDA graph)."""
         P = self.peer
-        bar = P["barrier"]
-        st = _lib.stream_ptr(stream)
-        if self.dp_signals:
-            _lib.check(self.lib.acez_adamw_dp_step(P["grads"], P["flags"], P["w16"], P["w3h"], P["params"], P["world"], P["rank"],
-                                                   self.n_params, _lib.ptr(P["reduced"]), _lib.ptr(self.params), _lib.ptr(self.exp_avg),
-                                                   _lib.ptr(self.exp_avg_sq), _lib.ptr(self.hyper), _lib.ptr(self.scaler_state),
-                                                   _lib.ptr(self.found_inf), C.c_void_p(self.grads_full.data_ptr() + 4 * self.n_params),
-                                                   _lib.ptr(self.dp_sync_state), _lib.ptr(self.stats), self.dp_multicast, self.L, self.C3, st),
-                       "acez_adamw_dp_step")
-            return
-        bar.barrier(channel=0)
-        _lib.check(self.lib.acez_adamw_dp_reduce(P["grads"], P["flags"], P["world"], P["rank"], self.n_params,
-                                                 _lib.ptr(P["reduced"]), st), "acez_adamw_dp_reduce")
-        bar.barrier(channel=1)
-        _lib.check(self.lib.acez_adamw_dp_apply(P["w16"], P["w3h"], P["params"], P["world"], P["rank"], self.n_params,
-                                                _lib.ptr(P["reduced"]), _lib.ptr(self.params), _lib.ptr(self.exp_avg),
-                                                _lib.ptr(self.exp_avg_sq), _lib.ptr(self.hyper), _lib.ptr(self.scaler_state),
-                                                _lib.ptr(self.dp_flags), _lib.ptr(self.found_inf),
-                                                C.c_void_p(self.grads_full.data_ptr() + 4 * self.n_params), self.L, self.C3, st),
-                   "acez_adamw_dp_apply")
-        bar.barrier(channel=2)
+        _lib.check(self.lib.acez_adamw_dp_step(P["grads"], P["flags"], P["w16"], P["w3h"], P["params"], P["world"], P["rank"],
+                                               self.n_params, _lib.ptr(P["reduced"]), _lib.ptr(self.params), _lib.ptr(self.exp_avg),
+                                               _lib.ptr(self.exp_avg_sq), _lib.ptr(self.hyper), _lib.ptr(self.scaler_state),
+                                               _lib.ptr(self.found_inf), C.c_void_p(self.grads_full.data_ptr() + 4 * self.n_params),
+                                               _lib.ptr(self.dp_sync_state), _lib.ptr(self.stats), self.dp_multicast, self.L, self.C3,
+                                               _lib.stream_ptr(stream)),
+                   "acez_adamw_dp_step")
 
     def gather_params_from_shards(self):
         """fp32 master weights live on their owner rank during peer-memory training: collect them on every rank (export)."""
@@ -334,7 +319,7 @@ class HeadEngine:
 
     def adamw_step(self, use_scaler=True, flag_complete=True, stream=None, check_flag_slot=False):
         """flag_complete: found_inf already covers all gradients (true after train_fwd_bwd).
-        check_flag_slot (data parallel, experimental): the check pass also covers grads_full[n_params], the slot the ranks'
+        check_flag_slot (data parallel through NCCL): the check pass also covers grads_full[n_params], the slot the ranks'
         local flags travelled in (+inf when set), so no separate unpack kernels are needed."""
         rc = self.lib.acez_adamw_step(_lib.ptr(self.params), _lib.ptr(self.grads), _lib.ptr(self.exp_avg),
                                       _lib.ptr(self.exp_avg_sq), self.n_params, _lib.ptr(self.hyper),

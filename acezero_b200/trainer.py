@@ -155,17 +155,10 @@ class TrainLoop:
         self._warm = 0
         self._refine_graphs = {}
         self._refine_warm = {}
-        import os
-        # the post-all-reduce check pass also reads the flag slot behind the gradient (no separate unpack kernels; validated at
-        # N = 2 in round 2)
-        self._dp_fused_flag = world_size > 1 and os.environ.get("ACEZ_DP_FUSED_FLAG", "1") != "0"
         # peer-memory optimiser (csrc/adamw_dp.cu) when the head was created over symmetric memory (HeadEngine(peer_group=...))
         self._dp_peers = world_size > 1 and getattr(head, "_symm", None) is not None and not self.refining
         if self._dp_peers and head.peer is None:
             head.setup_peers()
-        # with the cross-GPU synchronisation inside the optimiser kernels (HeadEngine.dp_signals) the whole iteration is ONE graph;
-        # with torch's barrier kernels around them the optimiser stays eager unless ACEZ_DP_PEERS_GRAPH=1
-        self._dp_peers_graph = (self._dp_peers and getattr(head, "dp_signals", False)) or os.environ.get("ACEZ_DP_PEERS_GRAPH", "0") == "1"
         self._graph_host = None
         self._warm_host = 0
         self.set_buffer(buffer)
@@ -286,23 +279,18 @@ class TrainLoop:
                 self._enqueue_schedule()
         bt = self.batch
         # data parallel: the fp16-overflow check must see the SUMMED gradient (a per-rank partial can pass while the sum
-        # overflows), so the optimiser runs its own check pass; single GPU: the backward kernels' folded check is complete
+        # overflows), so the optimiser runs its own check pass, which also reads the flag slot behind the gradient (the ranks'
+        # local flags); single GPU: the backward kernels' folded check is complete
         flag_complete = self.world == 1
-        fused_flag = self.world > 1 and self._dp_fused_flag and self.use_scaler
         if part == "optimizer":
-            if self._dp_peers:
-                h.adamw_step_peers()
-                return
-            if self.world > 1 and not fused_flag:
-                self._dp_unpack_flag()
-            h.adamw_step(use_scaler=self.use_scaler, flag_complete=flag_complete, check_flag_slot=fused_flag)
+            h.adamw_step(use_scaler=self.use_scaler, flag_complete=flag_complete, check_flag_slot=self.world > 1)
             return
         h.train_fwd_bwd(self.b, lp, bt["target_px"], bt["intrinsics"], bt["intrinsics_inv"],
                         aug_inv=bt["aug_poses_inv"], pose_inv=bt["poses_inv"], P=P,
                         target_crds=bt["target_crds"] if self.use_depth else None, features=None, d_P=d_P,
                         d_Kdiag=d_Kdiag, use_device_scale=True, use_device_loss_weight=True)
-        if self.world > 1 and not (self._dp_peers and getattr(h, "dp_signals", False)):
-            self._dp_pack_flag()   # (the peer-memory optimiser with in-kernel signalling packs the spare slots itself)
+        if self.world > 1 and not self._dp_peers:
+            self._dp_pack_flag()   # (the peer-memory optimiser packs the spare slots itself)
         if part == "fwd_bwd":
             return
         if self._dp_peers:
@@ -310,9 +298,7 @@ class TrainLoop:
             return
         if self.world > 1:
             self._dp_allreduce()
-            if not fused_flag:
-                self._dp_unpack_flag()
-        h.adamw_step(use_scaler=self.use_scaler, flag_complete=flag_complete, check_flag_slot=fused_flag)
+        h.adamw_step(use_scaler=self.use_scaler, flag_complete=flag_complete, check_flag_slot=self.world > 1)
 
     def _enqueue_schedule(self):
         """First kernel of the iteration: device-side lr / loss weight / cool-down trigger (csrc/schedule.cu). It books the
@@ -443,10 +429,6 @@ class TrainLoop:
         import torch.distributed as dist
         dist.all_reduce(self.head.grads_full)
 
-    def _dp_unpack_flag(self):
-        h = self.head
-        h.found_inf.copy_((h.grads_full[h.n_params:h.n_params + 1] != 0).to(torch.int32))
-
     def _dp_reduce_stats(self):
         """Global [loss sum, inlier count, valid count, non-finite flag]: the three sums travelled behind the gradient through
         the iteration's all-reduce (no extra collective); a non-finite loss on any rank makes the summed loss non-finite."""
@@ -505,9 +487,9 @@ class TrainLoop:
 
     def _step_on_static_batch(self, read_loss):
         """One iteration on whatever the static batch tensors hold (no gather); reads the loss statistics back."""
-        # (NCCL all-reduces are not captured: that data-parallel path runs eagerly; the peer-memory optimiser with in-kernel
-        # signalling is plain kernels on this stream and is captured like the single-GPU iteration)
-        if self.use_graph and (self.world == 1 or (self._dp_peers and self._dp_peers_graph)):
+        # (NCCL all-reduces are not captured: that data-parallel path runs eagerly; the peer-memory optimiser is plain kernels
+        # on this stream and is captured like the single-GPU iteration)
+        if self.use_graph and (self.world == 1 or self._dp_peers):
             if self._graph_host is None:
                 if self._warm_host < 2:
                     self._warm_host += 1
@@ -612,23 +594,13 @@ class TrainLoop:
                 self._warm += 1
                 self._enqueue_compute()
                 return
-            if self.world == 1:
+            if self.world == 1 or self._dp_peers:
+                # data parallel over peer memory: the optimiser kernels and their cross-GPU synchronisation are kernels on this
+                # stream, so the whole iteration is ONE graph, as on one GPU
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g):
                     self._enqueue_compute()
                 self._graph = (g,)
-            elif self._dp_peers and self._dp_peers_graph:
-                # data parallel over peer memory: the optimiser kernels and the cross-GPU barriers are kernels on this stream,
-                # so the whole iteration is ONE graph
-                g = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(g):
-                    self._enqueue_compute()
-                self._graph = (g,)
-            elif self._dp_peers:
-                ga = torch.cuda.CUDAGraph()
-                with torch.cuda.graph(ga):
-                    self._enqueue_compute(part="fwd_bwd")
-                self._graph = (ga, None)
             else:
                 # data parallel through NCCL: the all-reduce stays outside the graphs (two graphs around it)
                 ga, gb = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
@@ -639,9 +611,6 @@ class TrainLoop:
                 self._graph = (ga, gb)
         if len(self._graph) == 1:
             self._graph[0].replay()
-        elif self._graph[1] is None:
-            self._graph[0].replay()
-            self.head.adamw_step_peers()
         else:
             self._graph[0].replay()
             self._dp_allreduce()

@@ -80,14 +80,6 @@ typedef struct acez_gemm_desc {
 } acez_gemm_desc;
 
 int acez_gemm_f16(const acez_gemm_desc* d, acez_stream_t stream);
-/* EXPERIMENTAL probe (csrc/gemm2cta.cu; not used by any default path): the same GEMM with tcgen05 cta_group::2 — one cluster of
- * two CTAs per 256 x 256 tile, the B tile shared between the SM pair. fp32 epilogue (ACEZ_EPI_F32) only; operands both K-major
- * or both MN-major. Exists to validate the 2-CTA primitives the next versions of the weight-gradient GEMM and of the fused layer
- * chain are built on. */
-int acez_gemm2cta_f16(const acez_gemm_desc* d, acez_stream_t stream);
-/* Profiling probe (ACEZ_GEMM2_DBG=1): per-CTA cycle counters of the last acez_gemm2cta_f16 call, 8 slots per CTA:
- * [0] MMA warp waiting for operands, [1] MMA loop, [2] TMA producer waiting for free stages, [3] producer loop, [4] epilogue. */
-int acez_debug_gemm2_clocks(long long* host_out, size_t n_ctas);
 
 /* ------------------------------------------------------------------------------------------------------------
  * Fused reprojection loss + backward.
@@ -280,37 +272,28 @@ int acez_gather_rows_multi_sched(const void* const* srcs, void* const* dsts, con
 
 /* ------------------------------------------------------------------------------------------------------------
  * Data-parallel optimiser step over NVLink peer memory (G ranks of one box, one process per GPU): replaces "NCCL all-reduce
- * of the 8.4 MB gradient + replicated AdamW" with two kernels that read / write the other GPUs' buffers directly.
- * Rank r owns the parameter shard [r S, (r+1) S), S = acez_adamw_dp_shard(n, G).
- *   acez_adamw_dp_reduce  reduced_shard[i] = sum over ranks (in rank order) of peer_grads[q][r S + i]; the 4 spare floats
- *                         behind the gradient (+inf marker of the local GradScaler flag, loss / inlier / valid sums) are summed
- *                         into reduced_shard[S .. S+4); the fp16-range / inf verdict of the summed shard is OR-ed into slot
- *                         `rank` of EVERY rank's flag array (peer_flags[q], int[G], zero before the first step)
- *   -- cross-GPU barrier (the caller's: e.g. torch symmetric memory) --
- *   acez_adamw_dp_apply   found = any flag | non-finite marker; unless found: unscale + AdamW on the shard (params / moments of
- *                         this rank), the new weights rounded to fp16 and stored into EVERY rank's fp16 shadows (peer_w16 /
- *                         peer_w3h), the biases (the kernels read them in fp32) into every rank's parameters (peer_params); GradScaler.update(); the summed spare slots are copied to local_extras[0..4) (= this rank's
- *                         grads + n); my_flags cleared; *found_inf_dev = found
- *   -- cross-GPU barrier --
+ * of the 8.4 MB gradient + replicated AdamW" with kernels that read / write the other GPUs' buffers directly, synchronised
+ * across the GPUs inside the kernels (no caller barriers: the step is captured in ONE CUDA graph with the rest of the iteration).
+ * Rank r owns the parameter shard [r S, (r+1) S), S = acez_adamw_dp_shard(n, G). One step:
+ *   - reduce: sum over ranks of the gradient of this rank's shard; the 4 spare floats behind the gradient (+inf marker of the
+ *     local GradScaler flag, loss / inlier / valid sums) are summed too; the fp16-range / inf verdict of the summed shard goes to
+ *     EVERY rank
+ *   - apply: found = any rank's verdict | non-finite marker; unless found: unscale + AdamW on the shard (params / moments of
+ *     this rank), the new weights rounded to fp16 and stored into EVERY rank's fp16 shadows (peer_w16 / peer_w3h), the biases
+ *     (the kernels read them in fp32) into every rank's parameters (peer_params); GradScaler.update(); the summed spare slots are
+ *     copied to local_extras[0..4) (= this rank's grads + n); *found_inf_dev = found
  * peer_* are HOST arrays of G device pointers (peer mappings of the same buffer on every rank).
  * fp32 master weights and moments are valid on their owner rank only.
  * ---------------------------------------------------------------------------------------------------------- */
 size_t acez_adamw_dp_shard(size_t n, int world);
-int acez_adamw_dp_reduce(const void* const* peer_grads, void* const* peer_flags, int world, int rank, size_t n,
-                         float* reduced_shard, acez_stream_t stream);
-int acez_adamw_dp_apply(void* const* peer_w16, void* const* peer_w3h, void* const* peer_params, int world, int rank, size_t n,
-                        const float* reduced_shard, float* params, float* exp_avg, float* exp_avg_sq, const float* hyper_dev,
-                        float* scaler_state_dev, int* my_flags, int* found_inf_dev, float* local_extras, int L, int C3,
-                        acez_stream_t stream);
-/* Both kernels in one call with the cross-GPU synchronisation INSIDE them (no caller barriers, capturable in ONE CUDA graph with
- * the rest of the iteration): every rank's flag array must then hold 64 ints (zero before the first step): [0, G) the verdict
- * flags as above, [16, 16+G) / [24, 24+G) / [32, 32+G) epoch signals "gradient complete" / "shard reduced" / "weights written",
- * stored by the peers over NVLink (st.release.sys) and polled locally (ld.acquire.sys). sync_state_dev: unsigned[4] of this rank,
- * zero before the first step ([0] = completed steps, [1] = block counter). When the second kernel completes, every rank's shard
- * of the new weights has landed in this rank's buffers. A peer that never signals traps after ~20 s instead of hanging.
- * local_stats_dev (nullable): float[3] loss / inlier / valid sums of this rank's backward pass; when given, the first kernel packs
- * the four spare slots behind this rank's gradient itself (+inf marker from *found_inf_dev, then the three sums) and the step runs
- * as ONE kernel when the shard fits a co-resident grid's registers.
+/* Every rank's flag array (peer_flags) holds 64 ints, zero before the first step: [0, G) the verdict flags, [16, 16+G) /
+ * [24, 24+G) / [32, 32+G) epoch signals "gradient complete" / "shard reduced" / "weights written", stored by the peers over
+ * NVLink (st.release.sys) and polled locally (ld.acquire.sys). sync_state_dev: unsigned[4] of this rank, zero before the first
+ * step ([0] = completed steps, the rest block counters). When the call's last kernel completes, every rank's shard of the new
+ * weights has landed in this rank's buffers. A peer that never signals traps after ~20 s instead of hanging.
+ * local_stats_dev (nullable): float[3] loss / inlier / valid sums of this rank's backward pass; when given, the step packs the
+ * four spare slots behind this rank's gradient itself (+inf marker from *found_inf_dev, then the three sums) and runs as ONE
+ * kernel when the shard fits a co-resident grid's registers; otherwise (or without it) as a reduce kernel and an apply kernel.
  * multicast (nullable): host array of 4 NVSwitch multicast addresses of the gradient, fp16 hidden weights, fp16 fc3 weights and
  * parameter buffers (NVLink SHARP): the gradient is then summed inside the switch (multimem.ld_reduce) and the new weights reach
  * all ranks with one store each (multimem.st); the summation order inside the switch is the hardware's, every element is still

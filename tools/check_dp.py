@@ -79,39 +79,28 @@ def main():
             loop.train_iteration(perm[i * 5120 * world:(i + 1) * 5120 * world])
         torch.cuda.synchronize()
         dist.barrier()
-        if getattr(head, "dp_signals", False):
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                for _ in range(10):
-                    head.adamw_step_peers()
-            g.replay()
-            torch.cuda.synchronize()
-            dist.barrier()
-            e0, e1 = torch.cuda.Event(True), torch.cuda.Event(True)
-            e0.record()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
             for _ in range(10):
-                g.replay()
-            e1.record()
-            torch.cuda.synchronize()
-            us = e0.elapsed_time(e1) * 10.0   # ms / 100 steps -> us per step
-        else:
-            e0, e1 = torch.cuda.Event(True), torch.cuda.Event(True)
-            for _ in range(5):
                 head.adamw_step_peers()
-            e0.record()
-            for _ in range(100):
-                head.adamw_step_peers()
-            e1.record()
-            torch.cuda.synchronize()
-            us = e0.elapsed_time(e1) * 10.0
-        st = head.peer["reduced"][:16].view(torch.int64).cpu().numpy() if getattr(head, "dp_signals", False) else None
-        if rank == 0 and st is not None and st[0] > 0:
+        g.replay()
+        torch.cuda.synchronize()
+        dist.barrier()
+        e0, e1 = torch.cuda.Event(True), torch.cuda.Event(True)
+        e0.record()
+        for _ in range(10):
+            g.replay()
+        e1.record()
+        torch.cuda.synchronize()
+        us = e0.elapsed_time(e1) * 10.0   # ms / 100 steps -> us per step
+        st = head.peer["reduced"][:16].view(torch.int64).cpu().numpy()
+        if rank == 0 and st[0] > 0:
             d = [(int(st[i]) - int(st[0])) / 1000.0 for i in range(8)]
             print(f"[dp{world}] phases of the last fused optimiser kernel (us after its start, %globaltimer): gradients of all ranks ready {d[1]:.1f}, "
                   f"reduced + checked {d[2]:.1f}, global verdict {d[3]:.1f}, stored {d[4]:.1f}, block-0 fence {d[5]:.1f}, "
                   f"last block signalled {d[6]:.1f}, all ranks' weights landed {d[7]:.1f}")
         if rank == 0:
-            print(f"[dp{world}] optimiser step over peer memory alone (reduce + apply, {'in-kernel signals' if head.dp_signals else 'torch barriers'}): "
+            print(f"[dp{world}] optimiser step over peer memory alone (reduce + apply, in-kernel signals): "
                   f"{us:.1f} us per step (single-GPU AdamW kernel: ~16.5 us)")
         del loop, head
     merged = parallel.gather_registration(res, world)
