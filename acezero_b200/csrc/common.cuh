@@ -41,6 +41,47 @@ int make_tensor_map(CUtensorMap* out, CUtensorMapDataType dtype, int rank, const
 
 int sm_count();
 
+// Host: launch `kern` with clusters of CLUSTER CTAs along x (1: no cluster attribute). With `pdl` the launch carries the
+// programmatic-dependent-launch attribute: the kernel may be scheduled while its predecessor in the stream still runs; every
+// kernel launched this way starts with pdl_wait() (griddepcontrol.wait) before it touches global memory and calls
+// pdl_launch_dependents() so that ITS successor can be scheduled early in turn. The attribute is only safe when the stream
+// predecessor is a kernel: griddepcontrol.wait does not order against a preceding memcpy / memset / cross-stream event, so the
+// FIRST kernel of every C-ABI call is launched with pdl = false.
+template <int CLUSTER = 1, typename... KArgs, typename... Args>
+int launch_kernel(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool pdl, const Args&... args) {
+  cudaLaunchAttribute attr[2];
+  unsigned int n = 0;
+  if (CLUSTER > 1) {
+    attr[n].id = cudaLaunchAttributeClusterDimension;
+    attr[n].val.clusterDim.x = CLUSTER;
+    attr[n].val.clusterDim.y = 1;
+    attr[n].val.clusterDim.z = 1;
+    ++n;
+  }
+  if (pdl) {
+    attr[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[n].val.programmaticStreamSerializationAllowed = 1;
+    ++n;
+  }
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = grid;
+  cfg.blockDim = block;
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cfg.attrs = attr;
+  cfg.numAttrs = n;
+  ACEZ_CUDA(cudaLaunchKernelEx(&cfg, kern, args...));
+  return ACEZ_OK;
+}
+
+// Host: let kernel `Kern` use up to `bytes` of dynamic shared memory (more than 48 KB needs this opt-in). Only the first call
+// for a kernel reaches the runtime; later calls return its result.
+template <auto Kern>
+int set_max_dynamic_smem(int bytes) {
+  static const cudaError_t e = cudaFuncSetAttribute(Kern, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+  return e == cudaSuccess ? ACEZ_OK : cuda_fail(e, "cudaFuncSetAttribute(cudaFuncAttributeMaxDynamicSharedMemorySize)");
+}
+
 #ifdef __CUDACC__
 // ----------------------------------------------------------------------------------------------
 // device helpers

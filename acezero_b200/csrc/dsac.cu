@@ -373,12 +373,8 @@ extern "C" int acez_dsac_forward_rgb_batch(const float* sc, int n, int h, int w,
   a.stage_smem = 1;
   const size_t smem1 = (size_t)cells * 12;
   const size_t smem2 = smem1 + (size_t)cells * 2;
-  static bool configured = false;
-  if (!configured) {
-    ACEZ_CUDA(cudaFuncSetAttribute(dsac_sample_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-    ACEZ_CUDA(cudaFuncSetAttribute(dsac_refine_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 224 * 1024));
-    configured = true;
-  }
+  if ((rc = set_max_dynamic_smem<dsac_sample_score_kernel>(200 * 1024))) return rc;
+  if ((rc = set_max_dynamic_smem<dsac_refine_kernel>(224 * 1024))) return rc;
   ACEZ_REQUIRE(smem2 <= 224 * 1024, "dsac: %d cells exceed the refinement kernel's shared-memory budget", cells);
   const int warps = kDsacThreads / 32;
   // enough CTAs per image to fill the GPU when n is small; one chunk of 8 hypotheses per CTA pass

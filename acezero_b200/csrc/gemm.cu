@@ -435,26 +435,13 @@ int gemm_finalize(GemmLaunch* L) {
 
 template <int BN, bool A_MN, bool B_MN, int EPI>
 static int launch_variant(const GemmLaunch& L, cudaStream_t stream, bool pdl) {
-  auto kern = gemm_tcgen05_kernel<BN, A_MN, B_MN, EPI>;
-  static bool configured = false;
-  if (!configured) {
-    ACEZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, GemmCfg<BN, EPI>::kSmem));
-    configured = true;
-  }
+  constexpr auto kern = gemm_tcgen05_kernel<BN, A_MN, B_MN, EPI>;
+  int rc = set_max_dynamic_smem<kern>(GemmCfg<BN, EPI>::kSmem);
+  if (rc) return rc;
   dim3 grid((L.args.N + BN - 1) / BN, (L.args.M + BM - 1) / BM, L.batch);
   if (L.args.conv.enabled) grid.y = L.args.conv.tiles_x * L.args.conv.tiles_y * L.batch, grid.z = 1;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = dim3(kThreads);
-  cfg.dynamicSmemBytes = GemmCfg<BN, EPI>::kSmem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 1 : 0;
-  ACEZ_CUDA(cudaLaunchKernelEx(&cfg, kern, L.tmA, L.tmB, L.tmOut, L.tmOut2, L.tmOp, L.args));
-  return ACEZ_OK;
+  return launch_kernel(kern, grid, dim3(kThreads), GemmCfg<BN, EPI>::kSmem, stream, pdl, L.tmA, L.tmB, L.tmOut, L.tmOut2, L.tmOp,
+                       L.args);
 }
 
 int gemm_launch(const GemmLaunch& L, cudaStream_t stream, bool pdl) {

@@ -9,14 +9,9 @@
 //   * ITS HALF OF B (rows n0 + 128 r ..)     : 16 KB - the hardware feeds both tensor cores from both halves
 // i.e. 32 KB per CTA and k-block for 128 x 256 x 64 MACs per CTA: half the shared-memory fill and half the operand reads
 // per MAC of the cta_group::1 kernel with 128 x 128 tiles (round-1 measurement: the batched weight-gradient GEMM and the
-// fused layer chain are bound by the shared-memory port, DESIGN.md section 7). The 2-CTA primitives it uses (validated on
-// hardware in round 2; the layer chain of head_chain4.cu uses the same ones):
-//   - tcgen05.alloc / dealloc .cta_group::2 (same warp index in both CTAs, same destination offset)
-//   - cp.async.bulk.tensor .cta_group::2 : both CTAs' loads complete on the LEADER's (rank 0) full barrier (peer bit cleared)
-//   - tcgen05.mma.cta_group::2 issued by the leader's MMA warp only
-//   - tcgen05.commit.cta_group::2 ... multicast::cluster : stage release / accumulator-ready to BOTH CTAs
-// PTX forms follow the vendored CUTLASS headers (cute/arch/copy_sm100_tma.hpp, mma_sm100_umma.hpp,
-// tmem_allocator_sm100.hpp, cutlass/arch/barrier.h).
+// fused layer chain are bound by the shared-memory port, DESIGN.md section 7). The 2-CTA primitives (cluster2.cuh) are shared
+// with the layer chain of head_chain4.cu.
+#include "cluster2.cuh"
 #include "gemm2cta.cuh"
 
 namespace acez {
@@ -33,53 +28,6 @@ struct T2Cfg {
   static constexpr int kStage = T2_ASTAGE + kBStage;
   static constexpr int kSmem = T2_STAGES * kStage + 1024 /*ones tile*/ + 256 + 1024;
 };
-static constexpr uint32_t kPeerBitMask = 0xFEFFFFFFu;  // shared::cluster address of the same offset in the even CTA of the pair
-
-__device__ __forceinline__ uint32_t t2_cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void t2_cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void t2_tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "r"(ncols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void t2_tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// TMA load whose completion (bytes) is signalled on the LEADER CTA's barrier of the same offset
-__device__ __forceinline__ void t2_tma_load_3d(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
-          smem_u32(dst)),
-      "l"(map), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-// plain arrive on the leader's barrier (executed by the non-leader CTA)
-__device__ __forceinline__ void t2_arrive_leader(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & kPeerBitMask) : "memory");
-}
-__device__ __forceinline__ void t2_umma_f16(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-// arrive (once all prior UMMAs retire) on the barrier of this offset in BOTH CTAs of the pair
-__device__ __forceinline__ void t2_commit_both(uint64_t* bar, uint16_t mask = 0x3) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(mask)
-               : "memory");
-}
-
 // C4 = false: one CTA pair per 256 x BN tile (cluster of 2). C4 = true: cluster of FOUR CTAs = two pairs on the same tile, each
 // contracting half of the k-blocks into its own TMEM (split-K 2); pair B then ships its accumulator to pair A through
 // distributed shared memory (bulk copies into the drained pipeline stages) and pair A adds and stores: the reduction never
@@ -102,7 +50,7 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(free_bar + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int crank = (int)t2_cluster_ctarank();
+  const int crank = (int)cluster_ctarank();
   const int rank = crank & 1;               // CTA inside its pair
   const int kpair = C4 ? (crank >> 1) : 0;  // C4: 0 = pair A (first half of K, stores), 1 = pair B (second half, ships)
   const bool leader = rank == 0;
@@ -130,7 +78,7 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
     fence_barrier_init();
   }
   constexpr uint32_t kTmemCols = (T2_BN + 32 <= 256) ? 256u : 512u;  // accumulator + the bias-gradient column block
-  if (warp == 1) t2_tmem_alloc(tmem_ptr, kTmemCols);
+  if (warp == 1) tmem_alloc_pair(tmem_ptr, kTmemCols);
   // bias gradient dZ^T 1: one extra N = 16 UMMA per k-step against a ones tile (TMEM columns BN..BN+15). Every column tile of
   // an M-tile sees the same A operand, so the work is SPLIT over them: tile tn takes the k-blocks kb % tiles_n == tn (round 2
   // profile: with the whole column on the n0 == 0 tiles those CTAs ran 1.5x longer than the rest and set the kernel time);
@@ -144,7 +92,7 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
   }
   tcgen05_fence_before();
   __syncwarp();
-  t2_cluster_sync();
+  cluster_sync();
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   pdl_wait();               // the set-up above overlapped the predecessor's tail; its writes are visible from here on
@@ -162,20 +110,20 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         mbar_wait(&empty_bar[stage], phase ^ 1);
         if (args.dbg) t_wait += clock64() - t0;
         if (leader) mbar_arrive_expect_tx(&full_bar[stage], 2 * T2_STAGE);
-        else t2_arrive_leader(&full_bar[stage]);
+        else mbar_arrive_leader(&full_bar[stage]);
         uint8_t* a_dst = sA + stage * T2_ASTAGE;
         uint8_t* b_dst = sB + stage * T2_BSTAGE;
         if (A_MN) {
 #pragma unroll
-          for (int i = 0; i < T2_BM / 64; ++i) t2_tma_load_3d(a_dst + i * 8192, &tmA, &full_bar[stage], m0 + 64 * i, kb * T2_BK, z);
+          for (int i = 0; i < T2_BM / 64; ++i) tma_load_3d_pair(a_dst + i * 8192, &tmA, &full_bar[stage], m0 + 64 * i, kb * T2_BK, z);
         } else {
-          t2_tma_load_3d(a_dst, &tmA, &full_bar[stage], kb * T2_BK, m0, z);
+          tma_load_3d_pair(a_dst, &tmA, &full_bar[stage], kb * T2_BK, m0, z);
         }
         if (B_MN) {
 #pragma unroll
-          for (int i = 0; i < T2_BN / 128; ++i) t2_tma_load_3d(b_dst + i * 8192, &tmB, &full_bar[stage], nb0 + 64 * i, kb * T2_BK, z);
+          for (int i = 0; i < T2_BN / 128; ++i) tma_load_3d_pair(b_dst + i * 8192, &tmB, &full_bar[stage], nb0 + 64 * i, kb * T2_BK, z);
         } else {
-          t2_tma_load_3d(b_dst, &tmB, &full_bar[stage], kb * T2_BK, nb0, z);
+          tma_load_3d_pair(b_dst, &tmB, &full_bar[stage], kb * T2_BK, nb0, z);
         }
         if (++stage == T2_STAGES) { stage = 0; phase ^= 1; }
       }
@@ -206,18 +154,18 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         for (int k = 0; k < T2_BK / 16; ++k) {
           const uint64_t da = make_smem_desc(a_addr + k * args.a_kstep, args.a_lbo, args.a_sbo, 2);
           const uint64_t db = make_smem_desc(b_addr + k * args.b_kstep, args.b_lbo, args.b_sbo, 2);
-          t2_umma_f16(tmem_base, da, db, idesc, (kb != kb_begin || k != 0) ? 1u : 0u);
+          umma_f16_pair(tmem_base, da, db, idesc, (kb != kb_begin || k != 0) ? 1u : 0u);
           if (do_bias) {
             const uint64_t d1 = make_smem_desc(smem_u32(sOnes) + k * 32, 0, 1024, 2);
-            t2_umma_f16(tmem_base + T2_BN, da, d1, idesc_ones, (bias_started | (uint32_t)k) != 0u ? 1u : 0u);
+            umma_f16_pair(tmem_base + T2_BN, da, d1, idesc_ones, (bias_started | (uint32_t)k) != 0u ? 1u : 0u);
           }
         }
       }
       if (do_bias) bias_started = 1u;
       __syncwarp();
       if (elect_one()) {
-        t2_commit_both(&empty_bar[stage], pair_mask);
-        if (kb == kb_end - 1) t2_commit_both(tmem_full_bar, pair_mask);
+        tcgen05_commit_pair(&empty_bar[stage], pair_mask);
+        if (kb == kb_end - 1) tcgen05_commit_pair(tmem_full_bar, pair_mask);
       }
       __syncwarp();
       if (++stage == T2_STAGES) { stage = 0; phase ^= 1; }
@@ -270,16 +218,12 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
       if (warp == 2 && lane == 0) {
         mbar_wait(free_bar, 0);   // pair A has retired all its MMAs: its stages are free
         const uint32_t dst_rank = (uint32_t)(crank - 2);
-        uint32_t dst, bar;
-        asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(dst) : "r"(stg), "r"(dst_rank));
-        asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(bar) : "r"(smem_u32(part_bar)), "r"(dst_rank));
+        const uint32_t dst = mapa_cluster(stg, dst_rank);
+        const uint32_t bar = mapa_cluster(smem_u32(part_bar), dst_rank);
         constexpr uint32_t kChunk = 32 * kPitch;   // 4 copies of 32 rows + the bias rows
 #pragma unroll
-        for (uint32_t o = 0; o < T2_BM * kPitch; o += kChunk)
-          asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst + o),
-                       "r"(stg + o), "r"(kChunk), "r"(bar) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst + T2_BM * kPitch),
-                     "r"(stg + T2_BM * kPitch), "r"((uint32_t)(T2_BM * 4)), "r"(bar) : "memory");
+        for (uint32_t o = 0; o < T2_BM * kPitch; o += kChunk) dsmem_copy(dst + o, stg + o, kChunk, bar);
+        dsmem_copy(dst + T2_BM * kPitch, stg + T2_BM * kPitch, (uint32_t)(T2_BM * 4), bar);
       }
     } else {
       float bias_partner = 0.f;
@@ -287,9 +231,7 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
         // ---- pair A: arm the landing barrier, tell the partner that the stages are free, wait for its accumulator ----
         if (warp == 2 && lane == 0) {
           mbar_arrive_expect_tx(part_bar, kStageBytes);
-          uint32_t fb;
-          asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(fb) : "r"(smem_u32(free_bar)), "r"((uint32_t)(crank + 2)));
-          asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(fb) : "memory");
+          mbar_arrive_remote_release(mapa_cluster(smem_u32(free_bar), (uint32_t)(crank + 2)));
         }
         mbar_wait(part_bar, 0);
         if (grp == 0) {
@@ -386,40 +328,24 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
 
   __syncwarp();
   tcgen05_fence_before();
-  t2_cluster_sync();  // both tensor cores are done with both CTAs' shared memory and TMEM
+  cluster_sync();  // both tensor cores are done with both CTAs' shared memory and TMEM
   if (warp == 1) {
     tcgen05_fence_after();
-    t2_tmem_dealloc(tmem_base, kTmemCols);
+    tmem_dealloc_pair(tmem_base, kTmemCols);
   }
 }
 
 // MN-major operands (the weight gradient's dZ and X), 256-column tiles per CTA pair
 template <bool C4>
 static int launch2(const CUtensorMap& tmA, const CUtensorMap& tmB, const Gemm2Args& a, int batch, cudaStream_t stream, bool pdl) {
-  auto kern = gemm2cta_kernel<true, true, kGemm2BN, C4>;
+  constexpr auto kern = gemm2cta_kernel<true, true, kGemm2BN, C4>;
   constexpr int T2_SMEM = T2Cfg<kGemm2BN>::kSmem;
-  static bool configured = false;
-  if (!configured) {
-    ACEZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, T2_SMEM));
-    configured = true;
-  }
+  int rc = set_max_dynamic_smem<kern>(T2_SMEM);
+  if (rc) return rc;
+  constexpr int kCluster = C4 ? 4 : 2;   // CTAs per output tile
   const int tiles_m = (a.M + 2 * T2_BM - 1) / (2 * T2_BM);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((C4 ? 4 : 2) * tiles_m * a.tiles_n, 1, batch);
-  cfg.blockDim = dim3(T2_THREADS);
-  cfg.dynamicSmemBytes = T2_SMEM;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = C4 ? 4 : 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 2 : 1;
-  ACEZ_CUDA(cudaLaunchKernelEx(&cfg, kern, tmA, tmB, a));
-  return ACEZ_OK;
+  return launch_kernel<kCluster>(kern, dim3(kCluster * tiles_m * a.tiles_n, 1, batch), dim3(T2_THREADS), T2_SMEM, stream, pdl, tmA,
+                                 tmB, a);
 }
 
 int gemm2_launch(const Gemm2Launch& L, cudaStream_t s, bool pdl) {

@@ -11,7 +11,7 @@
 //   DZ             : [L][max_rows][512] fp16 gradient w.r.t. the pre-activation of each hidden layer (x grad_scale)
 //   GRES           : [max_rows][512] fp16 running skip-path gradient
 //   MASKB          : [L+1][max_rows][64 B] one bit per channel: ReLU masks written by the fused forward chain and read
-//                    by the fused dgrad chain (head_chain.cu); MASKB[l] belongs to ACT[l]
+//                    by the fused dgrad chain (head_chain4.cu); MASKB[l] belongs to ACT[l]
 #include <stdlib.h>
 
 #include <vector>
@@ -56,7 +56,7 @@ struct acez_head_plan {
   std::vector<acez::GemmLaunch> fwd;
   std::vector<acez::GemmLaunch> dgrad;
   acez::GemmLaunch wgrad;    // per-layer plans: all weight gradients in one cta_group::1 launch (grid.z = layer)
-  // fused layer chains (head_chain.cu): one launch for all hidden layers of a pass
+  // fused layer chains (head_chain4.cu): one launch for all hidden layers of a pass
   int use_chain;
   acez::ChainLaunch chain_fwd, chain_bwd;
   acez::Gemm2Launch wgrad2;  // chain plans: all weight gradients in one cta_group::2 launch (gemm2cta.cu)
@@ -89,27 +89,6 @@ static HeadLayout head_layout(const acez_head_config& cfg) {
   o.blkpart = off; off = align_up(off + 4096 * 8 * sizeof(float) + 4096, 1024);  // tail per-block partials + 1024 counters
   o.total = off;
   return o;
-}
-
-// Launch with the programmatic-dependent-launch attribute: the kernel may be scheduled while its predecessor in the
-// stream still runs; every kernel launched this way starts with pdl_wait() (griddepcontrol.wait) before it touches
-// global memory and calls pdl_launch_dependents() so that ITS successor can be scheduled early in turn.
-template <typename... KArgs, typename... Args>
-static int launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, bool pdl, Args... args) {
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = grid;
-  cfg.blockDim = block;
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  // The attribute is only safe when the stream predecessor is a kernel: griddepcontrol.wait does not order against a
-  // preceding memcpy / memset / cross-stream event, so the FIRST kernel of every C-ABI call is launched plainly.
-  cfg.numAttrs = pdl ? 1 : 0;
-  ACEZ_CUDA(cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...));
-  return ACEZ_OK;
 }
 
 // ----------------------------------------------------------------------------------------------
@@ -882,19 +861,16 @@ static int launch_tail(acez_head_plan* h, TailArgs& t, int rows, cudaStream_t s,
   t.blk_part = h->BLKPART;
   t.blk_count = h->BLKCOUNT;
   t.fc3_part = with_fc3_grad ? h->FC3PART : nullptr;
-  static bool configured = false;
-  if (!configured) {
-    ACEZ_CUDA(cudaFuncSetAttribute(head_tail_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTailAccBytes));
-    configured = true;
-  }
-  int rc = launch_pdl(head_tail_kernel, dim3(tail_grid(rows)), dim3(kTailThreads), with_fc3_grad ? (size_t)kTailAccBytes : 0, s, pdl, t);
+  int rc = set_max_dynamic_smem<head_tail_kernel>(kTailAccBytes);
+  if (rc) return rc;
+  rc = launch_kernel(head_tail_kernel, dim3(tail_grid(rows)), dim3(kTailThreads), with_fc3_grad ? (size_t)kTailAccBytes : 0, s, pdl, t);
   if (rc) return rc;
   if (with_fc3_grad) {
     const int nblk = tail_grid(rows);
     float* gW3 = h->grads + (size_t)h->L * kLayerStride;
     const int total = 4 * kC + 4;
-    rc = launch_pdl(fc3_reduce_kernel, dim3((total * 8 + 255) / 256), dim3(256), 0, s, true, (const float*)h->FC3PART, nblk, h->C3, gW3,
-                    gW3 + (size_t)h->C3 * kC, nonfinite);
+    rc = launch_kernel(fc3_reduce_kernel, dim3((total * 8 + 255) / 256), dim3(256), 0, s, true, (const float*)h->FC3PART, nblk, h->C3, gW3,
+                       gW3 + (size_t)h->C3 * kC, nonfinite);
     if (rc) return rc;
   }
   return ACEZ_OK;
@@ -987,7 +963,7 @@ extern "C" int acez_head_plan_create(const acez_head_config* cfg, float* params,
   h->BLKCOUNT = reinterpret_cast<unsigned int*>(base + lo.blkpart + 4096 * 8 * sizeof(float));
   h->counters_zeroed = false;
   {
-    // Default: all hidden layers of the forward / dgrad pass in one cluster kernel each (head_chain.cu); measured on
+    // Default: all hidden layers of the forward / dgrad pass in one cluster kernel each (head_chain4.cu); measured on
     // B200 (round 1, b = 5120): 0.212 ms per training iteration against 0.232 ms with one GEMM launch per layer.
     // ACEZ_HEAD_CHAIN=0 selects the per-layer tcgen05 GEMM path (also used when the head is deeper than the chain holds).
     const char* e = getenv("ACEZ_HEAD_CHAIN");
@@ -1179,8 +1155,8 @@ static int gather_multi_impl(const void* const* srcs, void* const* dsts, const i
   if (rows == 0) return ACEZ_OK;
   const int threads = 256;
   dim3 grid((rows * 32 + threads - 1) / threads + (sch.enabled ? 1 : 0));
-  return launch_pdl(gather_rows_multi_kernel, grid, dim3(threads), 0, reinterpret_cast<cudaStream_t>(stream), false, g, idx, rows,
-                    n_arrays, sch);
+  return launch_kernel(gather_rows_multi_kernel, grid, dim3(threads), 0, reinterpret_cast<cudaStream_t>(stream), false, g, idx, rows,
+                       n_arrays, sch);
 }
 
 extern "C" int acez_adamw_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, size_t n,
@@ -1197,12 +1173,12 @@ extern "C" int acez_adamw_step(float* params, const float* grads, float* exp_avg
   if (use_scaler == 1 || use_scaler == 3) {  // 2 = the caller's flag already covers every gradient (acez_head_train_fwd_bwd does)
     // 3 (data parallel through NCCL): one more element behind the gradient is checked too - the slot in which the ranks'
     // local GradScaler flags travelled through the all-reduce (+inf when any rank overflowed)
-    rc = launch_pdl(grad_check_kernel, dim3(grid), dim3(256), 0, s, false, grads, n + (use_scaler == 3 ? 1 : 0), found_inf_dev);
+    rc = launch_kernel(grad_check_kernel, dim3(grid), dim3(256), 0, s, false, grads, n + (use_scaler == 3 ? 1 : 0), found_inf_dev);
     if (rc) return rc;
   }
-  rc = launch_pdl(adamw_kernel, dim3(grid), dim3(256), 0, s, false, params, grads, exp_avg, exp_avg_sq, n, hyper_dev,
-                  scaler_state_dev, (const int*)found_inf_dev, use_scaler ? 1 : 0, plan ? plan->W16 : (__half*)nullptr,
-                  plan ? plan->W3h : (__half*)nullptr, plan ? plan->L : 0, plan ? plan->C3 : 0);
+  rc = launch_kernel(adamw_kernel, dim3(grid), dim3(256), 0, s, false, params, grads, exp_avg, exp_avg_sq, n, hyper_dev,
+                     scaler_state_dev, (const int*)found_inf_dev, use_scaler ? 1 : 0, plan ? plan->W16 : (__half*)nullptr,
+                     plan ? plan->W3h : (__half*)nullptr, plan ? plan->L : 0, plan ? plan->C3 : 0);
   if (rc) return rc;
   return ACEZ_OK;
 }

@@ -9,7 +9,7 @@
 // shared::cluster, completing on the partner's mbarrier), 64-column box by box, so the next layer's MMAs start while the
 // epilogue of the current one is still draining. Weights stream from L2 through a TMA ring that runs ahead across layer
 // boundaries. Every new activation tile is also written to HBM (TMA store) because the weight-gradient GEMM contracts over
-// ALL rows and stays a separate kernel. Kernel: head_chain4.cu; host side (tensor maps, dispatch): head_chain.cu.
+// ALL rows and stays a separate kernel. Kernel and host side: head_chain4.cu.
 #pragma once
 #include "common.cuh"
 
@@ -21,7 +21,9 @@ enum ChainMode : int { CHAIN_FWD = 0, CHAIN_DGRAD = 1 };
 // the clock is only read on the slow path, after a first failed try_wait.
 static constexpr long long kChainWatchdogCycles = 20000000000ll;
 static constexpr int kChainMaxSteps = 20;      // hidden layers handled by one launch (3 * res blocks + 2 <= 20)
-static constexpr int kChainFlagResInit = 64;   // ChainArgs.flags: FWD has residual layers, res_0 = the input tile
+static constexpr int kChainFlagResInit = 64;    // ChainArgs.flags: FWD has residual layers, res_0 = the input tile
+static constexpr int kChainFlagOwnFirst = 256;  // ChainArgs.flags: consume the own boxes' k-blocks first (default;
+                                                // ACEZ_CHAIN_ORDER=arrival clears it: they are consumed as they arrive)
 
 // One GEMM of the chain, in execution order.
 struct ChainStep {
@@ -41,9 +43,7 @@ static constexpr int kChainDbgSlots = 8 + 8 * kChainMaxSteps;  // clock64 stamps
 struct ChainArgs {
   int rows;
   int n_steps;
-  int flags;       // bit 0: relaxed (instead of release / acquire) cluster-scope signalling of the "A buffer free" barrier
-                   // bit 6 (kChainFlagResInit): see above
-                   // bit 8: consume the k-blocks own boxes first (default; ACEZ_CHAIN_ORDER=arrival clears it)
+  int flags;       // kChainFlagResInit | kChainFlagOwnFirst
   int* nonfinite;  // DGRAD: OR-ed with 1 if a stored gradient is inf / nan (nullable)
   long long* dbg;  // nullable: [gridDim.x][kChainDbgSlots] clock64 stamps (ACEZ_CHAIN_DBG=1, tools/probe_chain_time.py)
   ChainStep step[kChainMaxSteps];
@@ -51,11 +51,9 @@ struct ChainArgs {
 
 struct ChainLaunch {
   CUtensorMap tmIn;   // first A tile: [rows, 512], box {64, 128, 1}
-  CUtensorMap tmW;    // W16 [L][512][512]: FWD box {64, 256, 1} (K-major B), DGRAD box {64, 64, 1} (MN-major B); the kernel of
-                      // head_chain4.cu encodes its own map (each CTA of a pair stages half a k-block)
+  CUtensorMap tmW;    // W16 [L][512][512], half a k-block per CTA of a pair: FWD box {64, 128, 1} (K-major B), DGRAD box
+                      // {64, 64, 1} (MN-major B, two boxes per half)
   CUtensorMap tmOut;  // [slots][rows][512], box {64, 128, 1}
-  const __half* w16;  // the weight array and layer count the weight map is built from
-  int n_layers;
   ChainArgs args;
   int mode;
 };
@@ -65,9 +63,6 @@ int chain_prepare(ChainLaunch* C, int mode, const __half* in, const __half* W16,
                   long long out_zstride, int out_slots, int rows);
 // pdl: launch with the programmatic-dependent-launch attribute (only when the stream predecessor is a kernel)
 int chain_launch(const ChainLaunch& C, cudaStream_t stream, bool pdl = false);
-int chain4_launch(const ChainLaunch& C, cudaStream_t stream, bool pdl);  // the kernel launch (head_chain4.cu)
-// profiling probe: device buffer for the clock64 stamps of a launch with `ctas` CTAs (nullptr unless ACEZ_CHAIN_DBG=1)
-long long* chain_debug_buffer(int ctas);
 // profiling probe: copies the stamps of the most recent launch with ACEZ_CHAIN_DBG=1 to host memory
 int chain_debug_read(long long* host_out, size_t max_slots, int* n_ctas);
 

@@ -31,8 +31,10 @@
 //   * copy into the partner's box    after  peer_free phase s (= the partner's MMAs of step s retired)
 //   * TMEM buffer s&1 rewritten by MMA s+2: needs every box of epilogue s+1, which follows epilogue s in program order
 // The protocol is model-checked under random interleavings by tools/sim_chain4_protocol.py.
+// The host side (tensor maps of a pass, the launch, the profiling probe's stamp buffer) is at the end of this file.
 #include <stdlib.h>
 
+#include "cluster2.cuh"
 #include "head_chain.cuh"
 
 namespace acez {
@@ -47,45 +49,17 @@ static constexpr int kBStages = 6;
 static constexpr int kSmem4 = kABytes + kBStages * kBHalf + 1024 /*fp32 bias slice*/ + 384 /*barriers*/ + 1024 /*align*/;
 static_assert(kSmem4 <= 232448, "shared memory budget");
 static constexpr uint32_t kSw128 = 2;
-static constexpr uint32_t kPeerBit = 0xFEFFFFFFu;  // clears the pair bit of a shared::cluster address: the even CTA of the pair
 
-__device__ __forceinline__ uint32_t c4_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void c4_cluster_sync() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t c4_mapa(uint32_t addr, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void c4_arrive_remote_release(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ void c4_arrive_remote_relaxed(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.relaxed.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-__device__ __forceinline__ bool c4_try_wait(uint64_t* bar, uint32_t parity, int sem /*0 cta acquire, 1 cluster acquire, 2 cluster relaxed*/) {
+__device__ __forceinline__ bool c4_try_wait(uint64_t* bar, uint32_t parity, int sem /*0 cta acquire, 2 cluster relaxed*/) {
+  if (sem == 0) return mbar_try_wait(bar, parity);
   uint32_t ok;
-  if (sem == 0) {
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
-                 : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  } else if (sem == 1) {
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
-                 : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  } else {
-    asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.relaxed.cluster.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
-                 : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  }
+  asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.relaxed.cluster.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}\n"
+               : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
   return ok != 0;
 }
 __device__ __noinline__ void c4_timeout(uint32_t tag, uint32_t parity) {
   printf("acez: chain4 wait timeout: kind %u step %u index %u parity %u (block %d, cta rank %d, thread %d)\n", tag >> 16,
-         (tag >> 8) & 0xFF, tag & 0xFF, parity, blockIdx.x, (int)c4_ctarank(), threadIdx.x);
+         (tag >> 8) & 0xFF, tag & 0xFF, parity, blockIdx.x, (int)cluster_ctarank(), threadIdx.x);
   __trap();
 }
 // kinds: 1 a_ready, 2 b_full, 3 b_empty, 4 tmem_full, 5 peer_free, 7 partner_ready
@@ -97,46 +71,6 @@ __device__ __forceinline__ void c4_wait(uint64_t* bar, uint32_t parity, uint32_t
     if (clock64() - t0 > kChainWatchdogCycles) c4_timeout(tag, parity);
   }
 }
-__device__ __forceinline__ void c4_tmem_alloc(uint32_t* smem_dst, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "r"(ncols) : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void c4_tmem_dealloc(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// weight load of a CTA of the pair: completes (bytes) on the pair LEADER's barrier of the same offset
-__device__ __forceinline__ void c4_tma_load_pair(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
-          smem_u32(dst)),
-      "l"(map), "r"(smem_u32(bar) & kPeerBit), "r"(c0), "r"(c1), "r"(c2)
-      : "memory");
-}
-__device__ __forceinline__ void c4_arrive_leader(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & kPeerBit) : "memory");
-}
-__device__ __forceinline__ void c4_umma(uint32_t tmem_d, uint64_t da, uint64_t db, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n"
-      ".reg .pred p;\n"
-      "setp.ne.b32 p, %4, 0;\n"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n"
-      "}\n" ::"r"(tmem_d),
-      "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void c4_commit_pair(uint64_t* bar, uint16_t pair_mask) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(bar)),
-               "h"(pair_mask)
-               : "memory");
-}
-__device__ __forceinline__ void c4_dsmem_copy(uint32_t dst_cluster, uint32_t src_cta, uint32_t bytes, uint32_t mbar_cluster) {
-  asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_cluster),
-               "r"(src_cta), "r"(bytes), "r"(mbar_cluster)
-               : "memory");
-}
-__device__ __forceinline__ void c4_store_wait_read1() { asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory"); }
-
 // consumption order of the 8 k-blocks. Two epilogue groups publish own boxes 0,1 first and 2,3 one box time later, so the
 // ARRIVAL order is own 0,1 | exchange partner's 0,1 | own 2,3 | partner's 2,3. The alternative (own_first: own 0..3 | partner's
 // 0..3, the order of the cta_group::1 chain; four groups publish all own boxes together) sums the k-blocks in an order
@@ -242,7 +176,7 @@ head_chain4_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_consta
   uint32_t* tmem_ptr = reinterpret_cast<uint32_t*>(peer_free + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int rank = (int)c4_ctarank();
+  const int rank = (int)cluster_ctarank();
   const int c = rank >> 1, r = rank & 1;
   const bool leader = r == 0;
   const int xpeer = rank ^ 2;               // exchange partner: same row tile, other channel half
@@ -251,7 +185,7 @@ head_chain4_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_consta
   const int n_base = c * CN;                // the pair's output channels of every layer
   const int nb_half = n_base + r * (CN / 2);
   const int n_steps = args.n_steps;
-  const bool own_first = (args.flags & 256) != 0;   // k-block consumption order (default; ACEZ_CHAIN_ORDER=arrival clears it)
+  const bool own_first = (args.flags & kChainFlagOwnFirst) != 0;   // k-block consumption order
   long long* dbg = args.dbg != nullptr ? args.dbg + (size_t)blockIdx.x * kChainDbgSlots : nullptr;
 
   if (warp == 0 && lane == 0) {
@@ -271,10 +205,10 @@ head_chain4_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_consta
     mbar_init(peer_free, 1);
     fence_barrier_init();
   }
-  if (warp == 1) c4_tmem_alloc(tmem_ptr, 512);
+  if (warp == 1) tmem_alloc_pair(tmem_ptr, 512);
   tcgen05_fence_before();
   __syncwarp();
-  c4_cluster_sync();
+  cluster_sync();
   tcgen05_fence_after();
   const uint32_t tmem_base = *tmem_ptr;
   // programmatic dependent launch: everything above overlapped the predecessor's tail; its global writes are visible from
@@ -299,20 +233,20 @@ head_chain4_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_consta
           const int j = c4_order(i, c, own_first);
           c4_wait<0>(&b_empty[stage], phase ^ 1, (3u << 16) | ((uint32_t)s << 8) | (uint32_t)i);
           if (leader) mbar_arrive_expect_tx(&b_full[stage], 2 * kBHalf);
-          else c4_arrive_leader(&b_full[stage]);
+          else mbar_arrive_leader(&b_full[stage]);
           uint8_t* dst = sB + stage * kBHalf;
           if (!kDgrad) {
-            c4_tma_load_pair(dst, &tmW, &b_full[stage], j * CK, nb_half, wl);  // 128 weight rows x 64 input channels
+            tma_load_3d_pair(dst, &tmW, &b_full[stage], j * CK, nb_half, wl);  // 128 weight rows x 64 input channels
           } else {
 #pragma unroll
-            for (int t = 0; t < 2; ++t) c4_tma_load_pair(dst + t * 8192, &tmW, &b_full[stage], nb_half + 64 * t, j * CK, wl);
+            for (int t = 0; t < 2; ++t) tma_load_3d_pair(dst + t * 8192, &tmW, &b_full[stage], nb_half + 64 * t, j * CK, wl);
           }
           if (++stage == kBStages) { stage = 0; phase ^= 1; }
         }
       }
     }
   } else if (warp == 1) {
-    const uint32_t xpeer_free = c4_mapa(smem_u32(peer_free), (uint32_t)xpeer);
+    const uint32_t xpeer_free = mapa_cluster(smem_u32(peer_free), (uint32_t)xpeer);
     if (leader) {
       // ------------------------------ UMMA issuer (pair leader) ------------------------------
       constexpr uint32_t idesc = make_idesc_f16(2 * CM, CN, false, kDgrad);
@@ -337,20 +271,20 @@ head_chain4_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_consta
             for (int k = 0; k < CK / 16; ++k) {
               const uint64_t da = make_smem_desc(a_addr + k * 32, 0, 1024, kSw128);
               const uint64_t db = make_smem_desc(b_addr + k * b_kstep, b_lbo, 1024, kSw128);
-              c4_umma(d_tmem, da, db, idesc, (i | k) != 0 ? 1u : 0u);
+              umma_f16_pair(d_tmem, da, db, idesc, (i | k) != 0 ? 1u : 0u);
             }
           }
           __syncwarp();
           if (elect_one()) {
-            c4_commit_pair(&b_empty[stage], pair_mask);
-            if (i == kKB - 1) c4_commit_pair(&tmem_full[s & 1], pair_mask);
+            tcgen05_commit_pair(&b_empty[stage], pair_mask);
+            if (i == kKB - 1) tcgen05_commit_pair(&tmem_full[s & 1], pair_mask);
           }
           __syncwarp();
           if (++stage == kBStages) { stage = 0; phase ^= 1; }
         }
         c4_wait<0>(&tmem_full[s & 1], (uint32_t)((s >> 1) & 1), (4u << 16) | ((uint32_t)s << 8) | 1u);
         if (lane == 0) {
-          c4_arrive_remote_relaxed(xpeer_free);
+          mbar_arrive_remote_relaxed(xpeer_free);
           if (dbg) dbg[8 + 8 * s + 3] = clock64();
         }
         __syncwarp();
@@ -367,12 +301,12 @@ head_chain4_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_consta
             // async copies completed on the barrier) and it is my own tensor core that will read it: the signal to the
             // leader, which issues the UMMAs for both CTAs, carries no data - relaxed, no fence (a release at cluster scope
             // costs a MEMBAR.ALL.GPU per k-block here; measured ~600 cycles per handshake in the 2-CTA chain)
-            c4_arrive_remote_relaxed(c4_mapa(smem_u32(&partner_ready[j]), (uint32_t)(rank & ~1)));
+            mbar_arrive_remote_relaxed(mapa_cluster(smem_u32(&partner_ready[j]), (uint32_t)(rank & ~1)));
           }
           __syncwarp();
         }
         c4_wait<0>(&tmem_full[s & 1], (uint32_t)((s >> 1) & 1), (4u << 16) | ((uint32_t)s << 8) | 1u);
-        if (lane == 0) c4_arrive_remote_relaxed(xpeer_free);
+        if (lane == 0) mbar_arrive_remote_relaxed(xpeer_free);
         __syncwarp();
       }
     }
@@ -479,7 +413,7 @@ head_chain4_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_consta
           const uint32_t box_addr = smem_u32(sA + j * kBoxBytes);
           if (!last) {
             mbar_arrive(&a_ready[j]);
-            c4_dsmem_copy(c4_mapa(box_addr, (uint32_t)xpeer), box_addr, kBoxBytes, c4_mapa(smem_u32(&a_ready[j]), (uint32_t)xpeer));
+            dsmem_copy(mapa_cluster(box_addr, (uint32_t)xpeer), box_addr, kBoxBytes, mapa_cluster(smem_u32(&a_ready[j]), (uint32_t)xpeer));
           }
           if (st.out_slot >= 0) tma_store_3d(&tmOut, sA + j * kBoxBytes, n_base + b * 64, m0, st.out_slot);
           tma_store_commit();
@@ -496,47 +430,45 @@ head_chain4_kernel(const __grid_constant__ CUtensorMap tmIn, const __grid_consta
   if (dbg && threadIdx.x == 0) dbg[1] = clock64();
   __syncwarp();
   tcgen05_fence_before();
-  c4_cluster_sync();
+  cluster_sync();
   if (warp == 1) {
     tcgen05_fence_after();
-    c4_tmem_dealloc(tmem_base, 512);
+    tmem_dealloc_pair(tmem_base, 512);
   }
 }
 
-template <int MODE>
-static int chain4_launch_mode(const ChainLaunch& C, cudaStream_t stream, bool pdl) {
-  auto kern = head_chain4_kernel<MODE>;
-  static bool configured = false;
-  if (!configured) {
-    ACEZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem4));
-    configured = true;
-  }
-  // weight map of this variant: FWD box {64, 128, 1} (this CTA's half of a K-major weight k-block), DGRAD box {64, 64, 1}
-  CUtensorMap tmW4;
+// ----------------------------------------------------------------------------------------------
+// host side
+// ----------------------------------------------------------------------------------------------
+int chain_prepare(ChainLaunch* C, int mode, const __half* in, const __half* W16, int L, __half* out_base,
+                  long long out_zstride, int out_slots, int rows) {
+  ACEZ_REQUIRE(C && in && W16 && out_base && rows >= 1 && L >= 1 && out_slots >= 1, "chain_prepare: bad arguments");
+  C->mode = mode;
+  int rc;
   {
-    uint64_t dims[3] = {(uint64_t)kC, (uint64_t)kC, (uint64_t)C.n_layers};
-    uint64_t strides[2] = {(uint64_t)kC * 2, (uint64_t)kC * kC * 2};
-    uint32_t box[3] = {64, (uint32_t)(MODE == CHAIN_FWD ? CN / 2 : 64), 1};
-    int rc = make_tensor_map(&tmW4, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, C.w16, dims, strides, box, nullptr, CU_TENSOR_MAP_SWIZZLE_128B);
+    uint64_t dims[3] = {(uint64_t)kC, (uint64_t)rows, 1};
+    uint64_t strides[2] = {(uint64_t)kC * 2, (uint64_t)rows * kC * 2};
+    uint32_t box[3] = {64, (uint32_t)CM, 1};
+    rc = make_tensor_map(&C->tmIn, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, in, dims, strides, box, nullptr,
+                         CU_TENSOR_MAP_SWIZZLE_128B);
     if (rc) return rc;
   }
-  const int tiles = (C.args.rows + CM - 1) / CM;
-  const int clusters = (tiles + 1) / 2;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3(4 * clusters);
-  cfg.blockDim = dim3(320);
-  cfg.dynamicSmemBytes = kSmem4;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 4;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = pdl ? 2 : 1;
-  ChainArgs args = C.args;
+  {
+    uint64_t dims[3] = {(uint64_t)kC, (uint64_t)kC, (uint64_t)L};
+    uint64_t strides[2] = {(uint64_t)kC * 2, (uint64_t)kC * kC * 2};
+    uint32_t box[3] = {64, (uint32_t)(mode == CHAIN_FWD ? CN / 2 : 64), 1};
+    rc = make_tensor_map(&C->tmW, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, W16, dims, strides, box, nullptr,
+                         CU_TENSOR_MAP_SWIZZLE_128B);
+    if (rc) return rc;
+  }
+  {
+    uint64_t dims[3] = {(uint64_t)kC, (uint64_t)rows, (uint64_t)out_slots};
+    uint64_t strides[2] = {(uint64_t)kC * 2, (uint64_t)out_zstride * 2};
+    uint32_t box[3] = {64, (uint32_t)CM, 1};
+    rc = make_tensor_map(&C->tmOut, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, out_base, dims, strides, box, nullptr,
+                         CU_TENSOR_MAP_SWIZZLE_128B);
+    if (rc) return rc;
+  }
   static const bool own_first = [] {
     // default: own boxes first (the summation order closest to the per-layer kernels / the oracle; all parity tests hold
     // their round-1 tolerances). ACEZ_CHAIN_ORDER=arrival consumes the k-blocks as they arrive (measured 3 us / iteration
@@ -544,16 +476,59 @@ static int chain4_launch_mode(const ChainLaunch& C, cudaStream_t stream, bool pd
     const char* e = getenv("ACEZ_CHAIN_ORDER");
     return e == nullptr || e[0] != 'a';
   }();
-  if (own_first) args.flags |= 256;
-  args.dbg = chain_debug_buffer(4 * clusters);   // nullptr unless ACEZ_CHAIN_DBG=1 (tools/probe_chain_time.py)
-  ACEZ_CUDA(cudaLaunchKernelEx(&cfg, kern, C.tmIn, tmW4, C.tmOut, args));
+  C->args.rows = rows;
+  C->args.n_steps = 0;
+  C->args.flags = own_first ? kChainFlagOwnFirst : 0;
+  C->args.nonfinite = nullptr;
+  C->args.dbg = nullptr;
   return ACEZ_OK;
 }
 
-int chain4_launch(const ChainLaunch& C, cudaStream_t stream, bool pdl) {
-  ACEZ_REQUIRE(C.args.n_steps >= 1 && C.args.n_steps <= kChainMaxSteps, "chain4_launch: %d steps", C.args.n_steps);
-  if (C.mode == CHAIN_FWD) return chain4_launch_mode<CHAIN_FWD>(C, stream, pdl);
-  return chain4_launch_mode<CHAIN_DGRAD>(C, stream, pdl);
+static long long* g_chain_dbg = nullptr;
+static int g_chain_dbg_ctas = 0;
+static constexpr int kChainDbgMaxCtas = 1024;
+
+// profiling probe: device buffer for the clock64 stamps of a launch with `ctas` CTAs (nullptr unless ACEZ_CHAIN_DBG=1)
+static long long* chain_debug_buffer(int ctas) {
+  static const bool want_dbg = [] {
+    const char* e = getenv("ACEZ_CHAIN_DBG");
+    return e != nullptr && atoi(e) != 0;
+  }();
+  if (!want_dbg || ctas > kChainDbgMaxCtas) return nullptr;
+  if (g_chain_dbg == nullptr && cudaMalloc(&g_chain_dbg, (size_t)kChainDbgMaxCtas * kChainDbgSlots * sizeof(long long)) != cudaSuccess)
+    return nullptr;
+  g_chain_dbg_ctas = ctas;
+  return g_chain_dbg;
+}
+
+int chain_debug_read(long long* host_out, size_t max_slots, int* n_ctas) {
+  ACEZ_REQUIRE(host_out != nullptr && n_ctas != nullptr, "chain_debug_read: null argument");
+  *n_ctas = 0;
+  if (g_chain_dbg == nullptr) return ACEZ_OK;
+  ACEZ_CUDA(cudaDeviceSynchronize());
+  size_t n = (size_t)g_chain_dbg_ctas * kChainDbgSlots;
+  if (n > max_slots) n = max_slots;
+  ACEZ_CUDA(cudaMemcpy(host_out, g_chain_dbg, n * sizeof(long long), cudaMemcpyDeviceToHost));
+  *n_ctas = g_chain_dbg_ctas;
+  return ACEZ_OK;
+}
+
+template <int MODE>
+static int chain_launch_mode(const ChainLaunch& C, cudaStream_t stream, bool pdl) {
+  constexpr auto kern = head_chain4_kernel<MODE>;
+  int rc = set_max_dynamic_smem<kern>(kSmem4);
+  if (rc) return rc;
+  const int tiles = (C.args.rows + CM - 1) / CM;
+  const int ctas = 4 * ((tiles + 1) / 2);   // a cluster of four per two row tiles
+  ChainArgs args = C.args;
+  args.dbg = chain_debug_buffer(ctas);   // nullptr unless ACEZ_CHAIN_DBG=1 (tools/probe_chain_time.py)
+  return launch_kernel<4>(kern, dim3(ctas), dim3(320), kSmem4, stream, pdl, C.tmIn, C.tmW, C.tmOut, args);
+}
+
+int chain_launch(const ChainLaunch& C, cudaStream_t stream, bool pdl) {
+  ACEZ_REQUIRE(C.args.n_steps >= 1 && C.args.n_steps <= kChainMaxSteps, "chain_launch: %d steps", C.args.n_steps);
+  if (C.mode == CHAIN_FWD) return chain_launch_mode<CHAIN_FWD>(C, stream, pdl);
+  return chain_launch_mode<CHAIN_DGRAD>(C, stream, pdl);
 }
 
 }  // namespace acez

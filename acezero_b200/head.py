@@ -122,7 +122,7 @@ class HeadEngine:
 
     @property
     def fused_chain(self):
-        """True when the plan runs each pass over the hidden layers as one fused cluster kernel (head_chain.cu)."""
+        """True when the plan runs each pass over the hidden layers as one fused cluster kernel (head_chain4.cu)."""
         return bool(self.lib.acez_head_plan_fused_chain(self.plan))
 
     def chain_kernel_symbol(self):

@@ -150,12 +150,12 @@ int acez_head_sync_weights(acez_head_plan* plan, acez_stream_t stream);
 /* Device pointer of the plan's input activation buffer [max_rows,512] fp16 (gather target). */
 void* acez_head_input_ptr(acez_head_plan* plan);
 /* 1 if the plan runs all hidden layers of a pass (ace_network.py:120-136 and its autograd transpose) as ONE fused
- * cluster kernel per pass (csrc/head_chain.cu), 0 if it launches one tcgen05 GEMM per layer (csrc/gemm.cu). Both are
+ * cluster kernel per pass (csrc/head_chain4.cu), 0 if it launches one tcgen05 GEMM per layer (csrc/gemm.cu). Both are
  * sm_100a paths with identical semantics; the fused chain is the default, ACEZ_HEAD_CHAIN=0 at plan creation selects
  * the per-layer path. */
 int acez_head_plan_fused_chain(const acez_head_plan* plan);
 /* Profiling probe of the fused chain kernel (ACEZ_CHAIN_DBG=1): clock64 stamps of the most recent launch,
- * [n_ctas][8 + 8 * 20] (layout in csrc/head_chain.cu), copied to host memory. */
+ * [n_ctas][8 + 8 * 20] (layout in csrc/head_chain4.cu), copied to host memory. */
 int acez_debug_chain_clocks(long long* host_out, size_t max_slots, int* n_ctas);
 
 /* Forward only (registration; ace_network.py:120-149 under autocast): features -> scene coordinates.

@@ -1,4 +1,4 @@
-"""GPU parity of the fused layer-chain kernels (acezero_b200/csrc/head_chain.cu: all hidden layers of the forward /
+"""GPU parity of the fused layer-chain kernels (acezero_b200/csrc/head_chain4.cu: all hidden layers of the forward /
 dgrad pass in one cluster launch, tiles exchanged through distributed shared memory) against
 
   (a) the per-layer tcgen05 GEMM path (gemm.cu) on the same inputs -- same operands, same fp16 roundings, only the fp32

@@ -1,4 +1,4 @@
-"""Localise a mismatch of the fused layer-chain kernels (head_chain.cu) against the per-layer GEMM path.
+"""Localise a mismatch of the fused layer-chain kernels (head_chain4.cu) against the per-layer GEMM path.
 
 Runs one training forward + backward with both paths on the same inputs and prints, per layer buffer (ACT / XTRA / DZ)
 and per 64-column box, the worst relative difference -- so that a failure points at a role (own half vs. peer half of

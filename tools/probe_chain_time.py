@@ -59,43 +59,34 @@ def show(st, cta, n_steps, title):
 
 def main():
     bt = {k: v.to(dev) for k, v in ace_ref.synth_batch(5, B).items()}
-    # (relaxed handshake, unused): one combination; ACEZ_PROBE_COMBOS="0:0" times the release / acquire handshake instead
-    combos = [(1, 0)]
-    if os.environ.get("ACEZ_PROBE_COMBOS"):   # e.g. "1:0,1:16"
-        combos = [tuple(int(x) for x in c.split(":")) for c in os.environ["ACEZ_PROBE_COMBOS"].split(",")]
-    for relaxed, abl in combos:
-        os.environ["ACEZ_CHAIN_RELAXED"] = str(relaxed)
-        head = HeadEngine(1, True, (0, 0, 0), max_rows=B, training=True)
-        head.load_state(ace_ref.make_head_state(200, 1, True))
-        assert head.fused_chain
-        lib = head.lib
-        head.input_buffer(B).copy_(bt["features"])
-        lp = head.loss_params("dyntanh", 30.0, B)
+    head = HeadEngine(1, True, (0, 0, 0), max_rows=B, training=True)
+    head.load_state(ace_ref.make_head_state(200, 1, True))
+    assert head.fused_chain
+    lib = head.lib
+    head.input_buffer(B).copy_(bt["features"])
+    lp = head.loss_params("dyntanh", 30.0, B)
 
-        def fwd():
-            _lib.check(lib.acez_head_forward(head.plan, None, B, None, _lib.stream_ptr()))
+    def fwd():
+        _lib.check(lib.acez_head_forward(head.plan, None, B, None, _lib.stream_ptr()))
 
-        def full():
-            head.train_fwd_bwd(B, lp, bt["target_px"], bt["intrinsics"], bt["intrinsics_inv"], aug_inv=bt["aug_poses_inv"],
-                               pose_inv=bt["poses_inv"], use_device_scale=True)
+    def full():
+        head.train_fwd_bwd(B, lp, bt["target_px"], bt["intrinsics"], bt["intrinsics_inv"], aug_inv=bt["aug_poses_inv"],
+                           pose_inv=bt["poses_inv"], use_device_scale=True)
 
-        t_f = timeit(fwd)
-        t_a = timeit(full)
-        fwd()
-        torch.cuda.synchronize()
-        st = stamps(lib)
-        tot_f = st[:, 1] - st[:, 0]
-        st_f = st.copy()
-        full()
-        torch.cuda.synchronize()
-        st = stamps(lib)   # the last chain launch of `full` is the dgrad chain
-        tot_d = st[:, 1] - st[:, 0]
-        print(f"relaxed={relaxed} ablate={abl:2d}: forward chain {t_f:7.1f} us  fwd+tail+bwd {t_a:7.1f} us | median CTA cycles "
-              f"fwd {int(np.median(tot_f))} dgrad {int(np.median(tot_d))}", flush=True)
-        if True:
-            show(st_f, 0, head.L, "fwd")
-            show(st, 0, head.L - 1, "dgrad")
-        del head
+    t_f = timeit(fwd)
+    t_a = timeit(full)
+    fwd()
+    torch.cuda.synchronize()
+    st_f = stamps(lib)
+    tot_f = st_f[:, 1] - st_f[:, 0]
+    full()
+    torch.cuda.synchronize()
+    st = stamps(lib)   # the last chain launch of `full` is the dgrad chain
+    tot_d = st[:, 1] - st[:, 0]
+    print(f"forward chain {t_f:7.1f} us  fwd+tail+bwd {t_a:7.1f} us | median CTA cycles "
+          f"fwd {int(np.median(tot_f))} dgrad {int(np.median(tot_d))}", flush=True)
+    show(st_f, 0, head.L, "fwd")
+    show(st, 0, head.L - 1, "dgrad")
 
 
 if __name__ == "__main__":
