@@ -20,12 +20,10 @@
 //           waits for everybody's.
 // Traffic per GPU and iteration: (G-1)/G * 8.4 MB of gradient reads + (G-1)/G * 4.2 MB of weight writes over NVLink, AdamW
 // state traffic 1/G of the single-GPU kernel. fp32 master weights are valid on their owner only (gathered when exported).
-#include "common.cuh"
+#include "adamw.cuh"
 
 namespace acez {
 
-static constexpr int kC = 512;
-static constexpr size_t kLayerStride = (size_t)kC * kC + kC;
 static constexpr int kMaxRanks = 8;
 
 // Cross-GPU synchronisation INSIDE the kernels: every rank's flag array (symmetric memory, int[kDpFlagInts]) also carries three
@@ -64,6 +62,15 @@ __device__ __forceinline__ void dp_wait_row(const int* my_flags, int row, int q,
     }
   }
 }
+
+// The four spare slots behind each rank's flat gradient: [n] +inf if the rank's local backward overflowed (GradScaler flag), else 0;
+// [n+1 .. n+3] the loss / inlier / valid sums of its local backward pass. Summed over the ranks, the first slot is non-zero or not
+// finite when any rank overflowed.
+__device__ __forceinline__ void pack_spare_slots(float* my_grads, size_t n, const int* local_found_inf, const float* local_stats) {
+  my_grads[n] = (*local_found_inf != 0) ? __int_as_float(0x7f800000) : 0.f;
+  my_grads[n + 1] = local_stats[0]; my_grads[n + 2] = local_stats[1]; my_grads[n + 3] = local_stats[2];
+}
+__device__ __forceinline__ bool overflow_marked(float slot) { return !isfinite(slot) || slot != 0.f; }
 
 // NVLink SHARP (multicast objects of the NVSwitch, PTX multimem.*): one load returns the sum over all GPUs' copies of an address
 // (the reduction happens in the switch: a GPU receives 1/G of the gradient instead of reading (G-1)/G of it from its peers, which a
@@ -109,10 +116,7 @@ adamw_dp_reduce_kernel(const DpPeers P, int world, int rank, size_t n, size_t sh
   const int epoch = (int)sync_state[0] + 1;
   // this rank's gradient is complete (stream order / the wait above): pack the spare slots behind it (the +inf marker of the
   // local GradScaler flag, the loss / inlier / valid sums of the local backward pass), tell everybody, wait for everybody's
-  if (blockIdx.x == 0 && threadIdx.x == 0 && my_grads != nullptr) {
-    my_grads[n] = (*local_found_inf != 0) ? __int_as_float(0x7f800000) : 0.f;
-    my_grads[n + 1] = local_stats[0]; my_grads[n + 2] = local_stats[1]; my_grads[n + 3] = local_stats[2];
-  }
+  if (blockIdx.x == 0 && threadIdx.x == 0 && my_grads != nullptr) pack_spare_slots(my_grads, n, local_found_inf, local_stats);
   if (blockIdx.x == 0) {
     __syncthreads();
     if (threadIdx.x < world) {
@@ -147,7 +151,7 @@ adamw_dp_reduce_kernel(const DpPeers P, int world, int rank, size_t n, size_t sh
       for (int r = 0; r < kMaxRanks; ++r)   // fixed order: the sum does not depend on who computes it
         if (r < world) { s.x += g[u][r].x; s.y += g[u][r].y; s.z += g[u][r].z; s.w += g[u][r].w; }
       reinterpret_cast<float4*>(reduced)[q] = s;
-      // under autocast the weight gradient is materialised in fp16: |g| > 65504 overflows to inf there
+      // fp16_grad_overflow() of the four sums, written out: through the helper nvcc schedules this loop differently
       bad |= !isfinite(s.x) || fabsf(s.x) > 65504.f || !isfinite(s.y) || fabsf(s.y) > 65504.f;
       bad |= !isfinite(s.z) || fabsf(s.z) > 65504.f || !isfinite(s.w) || fabsf(s.w) > 65504.f;
     }
@@ -156,7 +160,7 @@ adamw_dp_reduce_kernel(const DpPeers P, int world, int rank, size_t n, size_t sh
     float s = 0.f;
     for (int r = 0; r < world; ++r) s += __ldcg(P.grads[r] + i);
     reduced[i - lo] = s;
-    bad |= !isfinite(s) || fabsf(s) > 65504.f;
+    bad |= fp16_grad_overflow(s);
   }
   if (blockIdx.x == 0 && threadIdx.x < 4) {   // the spare slots: every rank for itself (all ranks get the same sums)
     float s = 0.f;
@@ -189,24 +193,12 @@ __global__ void adamw_dp_apply_kernel(const DpPeers P, int world, int rank, size
   int found = 0;
   for (int r = 0; r < world; ++r) found |= my_flags[r];
   const float flag_slot = reduced[shard];    // sum of the ranks' +inf markers (local backward overflow)
-  if (!isfinite(flag_slot) || flag_slot != 0.f) found = 1;
+  if (!isfinite(flag_slot) || flag_slot != 0.f) found = 1;   // overflow_marked(), written out: nvcc compiles the helper differently here
   const size_t lo = (size_t)rank * shard;
   const size_t hi = lo + shard < n ? lo + shard : n;
   if (!found) {
-    const float lr = hyper[0], b1 = hyper[1], b2 = hyper[2], eps = hyper[3], wd = hyper[4];
-    const float inv_scale = 1.f / scaler_state[0];
-    const float t = scaler_state[2] + 1.f;
-    const float bc1 = 1.f - powf(b1, t), bc2 = 1.f - powf(b2, t);
-    const float step_size = lr / bc1;
-    const float bc2_sqrt = sqrtf(bc2);
+    const AdamWStep adamw(hyper, scaler_state, true);
     const size_t wsz = (size_t)kC * kC;
-    auto update = [&](float gi, float& pi, float& mi, float& vi) {
-      gi = __half2float(__float2half_rn(gi)) * inv_scale;   // fp16 weight gradient of the autocast conv, GradScaler.unscale_
-      pi *= (1.f - lr * wd);
-      mi = mi + (1.f - b1) * (gi - mi);
-      vi = b2 * vi + (1.f - b2) * gi * gi;
-      pi -= step_size * (mi / (sqrtf(vi) / bc2_sqrt + eps));
-    };
     // groups of 8 consecutive parameters (shard bounds, layer strides and the weight / bias boundaries are multiples of 8): the
     // fp16 shadow travels to every rank as ONE 16-byte store per group and peer
     const size_t n8 = hi > lo ? (hi - lo) / 8 : 0;
@@ -222,7 +214,7 @@ __global__ void adamw_dp_apply_kernel(const DpPeers P, int world, int rank, size
       *reinterpret_cast<float4*>(v8) = *reinterpret_cast<const float4*>(v + i);
       *reinterpret_cast<float4*>(v8 + 4) = *reinterpret_cast<const float4*>(v + i + 4);
 #pragma unroll
-      for (int k = 0; k < 8; ++k) update(g8[k], p8[k], m8[k], v8[k]);
+      for (int k = 0; k < 8; ++k) adamw.update(g8[k], p8[k], m8[k], v8[k]);
       *reinterpret_cast<float4*>(p + i) = *reinterpret_cast<float4*>(p8);
       *reinterpret_cast<float4*>(p + i + 4) = *reinterpret_cast<float4*>(p8 + 4);
       *reinterpret_cast<float4*>(m + i) = *reinterpret_cast<float4*>(m8);
@@ -256,7 +248,7 @@ __global__ void adamw_dp_apply_kernel(const DpPeers P, int world, int rank, size
     }
     for (size_t i = lo + 8 * n8 + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < hi; i += (size_t)gridDim.x * blockDim.x) {
       float pi = p[i], mi = m[i], vi = v[i];
-      update(reduced[i - lo], pi, mi, vi);
+      adamw.update(reduced[i - lo], pi, mi, vi);
       p[i] = pi; m[i] = mi; v[i] = vi;
       const size_t l = i / kLayerStride, r = i % kLayerStride;
       const __half hv = __float2half_rn(pi);
@@ -280,12 +272,7 @@ __global__ void adamw_dp_apply_kernel(const DpPeers P, int world, int rank, size
     __threadfence_system();   // this block's remote weight stores before its arrival
     unsigned int* cnt = reinterpret_cast<unsigned int*>(scaler_state + 3);
     if (atomicAdd(cnt, 1u) == gridDim.x - 1) {
-      if (found) { scaler_state[0] *= 0.5f; scaler_state[1] = 0.f; }
-      else {
-        scaler_state[2] += 1.f;
-        scaler_state[1] += 1.f;
-        if (scaler_state[1] >= 2000.f) { scaler_state[0] *= 2.f; scaler_state[1] = 0.f; }
-      }
+      scaler_update(scaler_state, found, 1);
       *found_inf_out = found;
       for (int r = 0; r < world; ++r) my_flags[r] = 0;   // every block has read them (this is the last block to get here)
       *cnt = 0u;
@@ -334,8 +321,7 @@ adamw_dp_fused_kernel(const DpPeers P, int world, int rank, size_t n, size_t sha
   // ---- 1: gradient complete ----
   if (blockIdx.x == 0) {
     if (threadIdx.x == 0) {
-      my_grads[n] = (*found_inf_io != 0) ? __int_as_float(0x7f800000) : 0.f;
-      my_grads[n + 1] = local_stats[0]; my_grads[n + 2] = local_stats[1]; my_grads[n + 3] = local_stats[2];
+      pack_spare_slots(my_grads, n, found_inf_io, local_stats);
       __threadfence_system();   // ONE system-scope fence, then plain signal stores (the gradient itself is complete by stream order)
       for (int r = 0; r < world; ++r) st_relaxed_sys(P.flags[r] + kSigGrads + rank, epoch);
     }
@@ -405,7 +391,7 @@ adamw_dp_fused_kernel(const DpPeers P, int world, int rank, size_t n, size_t sha
         for (int r = 0; r < MAXW; ++r)   // fixed order: the sum does not depend on who computes it
           if (r < wsum) sum += gr[k][r][e];
         g8[k][e] = sum;
-        bad |= !isfinite(sum) || fabsf(sum) > 65504.f;   // the autocast weight gradient is fp16: beyond its range = inf
+        bad |= fp16_grad_overflow(sum);
       }
     }
     if (blockIdx.x == 0 && threadIdx.x >= 32 && threadIdx.x < 36) {   // the spare slots: every rank for itself (same sums everywhere)
@@ -430,27 +416,14 @@ adamw_dp_fused_kernel(const DpPeers P, int world, int rank, size_t n, size_t sha
   }
   // ---- 4: AdamW in registers, then the global verdict ----
   {
-    const float lr = hyper[0], b1 = hyper[1], b2 = hyper[2], eps = hyper[3], wd = hyper[4];
-    const float inv_scale = 1.f / scaler_state[0];
-    const float t = scaler_state[2] + 1.f;
-    const float bc1 = 1.f - powf(b1, t), bc2 = 1.f - powf(b2, t);
-    const float step_size = lr / bc1;
-    const float bc2_sqrt = sqrtf(bc2);
+    const AdamWStep adamw(hyper, scaler_state, true);
 #pragma unroll
-    for (int k = 0; k < GPT; ++k) {
+    for (int k = 0; k < GPT; ++k)
 #pragma unroll
-      for (int e = 0; e < 8; ++e) {
-        float gi = __half2float(__float2half_rn(g8[k][e])) * inv_scale;   // fp16 weight gradient of the autocast conv, unscale_
-        float pi = p8[k][e] * (1.f - lr * wd);
-        const float mi = m8[k][e] + (1.f - b1) * (gi - m8[k][e]);
-        const float vi = b2 * v8[k][e] + (1.f - b2) * gi * gi;
-        pi -= step_size * (mi / (sqrtf(vi) / bc2_sqrt + eps));
-        p8[k][e] = pi; m8[k][e] = mi; v8[k][e] = vi;
-      }
-    }
+      for (int e = 0; e < 8; ++e) adamw.update(g8[k][e], p8[k][e], m8[k][e], v8[k][e]);
   }
   int found_t = 0;
-  if (mc && threadIdx.x == 0) found_t = (!isfinite(marker) || marker != 0.f) ? 1 : 0;
+  if (mc && threadIdx.x == 0) found_t = overflow_marked(marker) ? 1 : 0;
   if (threadIdx.x < world) {
     const int* sp = my_flags + kSigReduced + threadIdx.x;
     int val = ld_acquire_sys(sp);
@@ -464,7 +437,7 @@ adamw_dp_fused_kernel(const DpPeers P, int world, int rank, size_t n, size_t sha
         }
       }
     }
-    found_t |= (val & 1) | ((!isfinite(marker) || marker != 0.f) ? 1 : 0);
+    found_t |= (val & 1) | (overflow_marked(marker) ? 1 : 0);
   }
   const int found = __syncthreads_or(found_t);
   if (stamp0) stamps[3] = now();
@@ -534,12 +507,7 @@ adamw_dp_fused_kernel(const DpPeers P, int world, int rank, size_t n, size_t sha
     if (stamp0) stamps[5] = now();
     if (atomicAdd(sync_state + 3, 1u) == gridDim.x - 1) {
       sync_state[3] = 0u;
-      if (found) { scaler_state[0] *= 0.5f; scaler_state[1] = 0.f; }
-      else {
-        scaler_state[2] += 1.f;
-        scaler_state[1] += 1.f;
-        if (scaler_state[1] >= 2000.f) { scaler_state[0] *= 2.f; scaler_state[1] = 0.f; }
-      }
+      scaler_update(scaler_state, found, 1);
       *found_inf_io = found;
       for (int k = 0; k < 4; ++k) my_grads[n + k] = scratch[k];   // every rank has read this rank's slots (its verdict came after)
       sync_state[0] = (unsigned int)epoch;
@@ -551,24 +519,6 @@ adamw_dp_fused_kernel(const DpPeers P, int world, int rank, size_t n, size_t sha
       stamps[7] = now();
     }
   }
-}
-
-template <int GPT, int MAXW>
-static int launch_fused(const DpPeers& P, int world, int rank, size_t n, size_t shard, float* p, float* m, float* v, const float* hyper,
-                        float* scaler_state, int* found_inf, float* my_grads, const float* local_stats, float* scratch,
-                        unsigned int* sync_state, unsigned long long* stamps, int L, int C3, cudaStream_t st, bool* launched) {
-  auto kern = adamw_dp_fused_kernel<GPT, MAXW>;
-  int per_sm = 0;
-  ACEZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, 0));
-  if (per_sm > 2) per_sm = 2;
-  const size_t n8 = (shard + 7) / 8;
-  const size_t threads = (size_t)per_sm * sm_count() * 256;
-  *launched = per_sm >= 1 && n8 <= (size_t)GPT * threads;
-  if (!*launched) return ACEZ_OK;
-  kern<<<per_sm * sm_count(), 256, 0, st>>>(P, world, rank, n, shard, p, m, v, hyper, scaler_state, found_inf, my_grads, local_stats,
-                                            scratch, sync_state, stamps, L, C3);
-  ACEZ_CUDA(cudaGetLastError());
-  return ACEZ_OK;
 }
 
 }  // namespace acez
@@ -591,7 +541,7 @@ extern "C" int acez_adamw_dp_step(const void* const* peer_grads, void* const* pe
                "adamw_dp_step: null argument");
   ACEZ_REQUIRE(world >= 1 && world <= kMaxRanks && rank >= 0 && rank < world && L >= 1 && (C3 == 3 || C3 == 4),
                "adamw_dp_step: bad arguments");
-  ACEZ_REQUIRE(n == (size_t)L * kLayerStride + (size_t)C3 * kC + (size_t)C3, "adamw_dp_step: parameter count does not match the head");
+  ACEZ_REQUIRE(n == head_param_count(L, C3), "adamw_dp_step: parameter count does not match the head");
   int rc = acez_device_check();
   if (rc) return rc;
   DpPeers P{};
@@ -612,15 +562,19 @@ extern "C" int acez_adamw_dp_step(const void* const* peer_grads, void* const* pe
   const size_t shard = acez_adamw_dp_shard(n, world);
   cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
   if (local_stats_dev != nullptr) {
-    // the one-kernel step (the shard's parameter groups fit the registers of one co-resident grid); scratch = the four floats
-    // behind the reduced-shard buffer
-    bool launched = false;
-    float* my_grads = local_extras - n;
-    if (world <= 2) rc = launch_fused<2, 2>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
-    else if (world <= 4) rc = launch_fused<1, 4>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
-    else rc = launch_fused<1, 8>(P, world, rank, n, shard, params, exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, my_grads, local_stats_dev, reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3, st, &launched);
-    if (rc) return rc;
-    if (launched) return ACEZ_OK;
+    // the one-kernel step, when the shard's parameter groups (gpt per thread) fit the registers of one co-resident grid; scratch =
+    // the four floats behind the reduced-shard buffer. Launched plainly (no programmatic dependent launch): the grid starts only
+    // after the previous kernel of the stream has drained, so all of it is resident.
+    const int gpt = world <= 2 ? 2 : 1;
+    const auto kern = world <= 2 ? &adamw_dp_fused_kernel<2, 2> : world <= 4 ? &adamw_dp_fused_kernel<1, 4> : &adamw_dp_fused_kernel<1, 8>;
+    int per_sm = 0;
+    ACEZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, 0));
+    if (per_sm > 2) per_sm = 2;
+    const size_t threads = (size_t)per_sm * sm_count() * 256;
+    if (per_sm >= 1 && (shard + 7) / 8 <= (size_t)gpt * threads)
+      return launch_kernel(kern, dim3(per_sm * sm_count()), dim3(256), 0, st, false, P, world, rank, n, shard, params, exp_avg,
+                           exp_avg_sq, hyper_dev, scaler_state_dev, found_inf_dev, local_extras - n, local_stats_dev,
+                           reduced_shard + shard, sync_state_dev, reinterpret_cast<unsigned long long*>(reduced_shard), L, C3);
   }
   // (blocks that poll a signal wait for REMOTE progress only, and the signals are sent by block 0 / the last block to finish:
   // no block of these grids waits for another block of its own GPU, so residency is not a correctness condition)
@@ -628,11 +582,10 @@ extern "C" int acez_adamw_dp_step(const void* const* peer_grads, void* const* pe
   // local_extras = this rank's gradient + n: the four spare slots; local_stats_dev (nullable): pack them here instead of in
   // separate kernels (found_inf_dev still holds the local backward's flag at this point)
   float* my_grads = local_stats_dev != nullptr ? local_extras - n : nullptr;
-  adamw_dp_reduce_kernel<<<grid, 256, 0, st>>>(P, world, rank, n, shard, reduced_shard, my_grads, found_inf_dev, local_stats_dev,
-                                               sync_state_dev);
-  ACEZ_CUDA(cudaGetLastError());
-  adamw_dp_apply_kernel<<<grid, 256, 0, st>>>(P, world, rank, n, shard, reduced_shard, params, exp_avg, exp_avg_sq, hyper_dev,
-                                              scaler_state_dev, P.flags[rank], found_inf_dev, local_extras, L, C3, sync_state_dev);
-  ACEZ_CUDA(cudaGetLastError());
-  return ACEZ_OK;
+  rc = launch_kernel(adamw_dp_reduce_kernel, dim3(grid), dim3(256), 0, st, false, P, world, rank, n, shard, reduced_shard, my_grads,
+                     found_inf_dev, local_stats_dev, sync_state_dev);
+  if (rc) return rc;
+  return launch_kernel(adamw_dp_apply_kernel, dim3(grid), dim3(256), 0, st, false, P, world, rank, n, shard, reduced_shard, params,
+                       exp_avg, exp_avg_sq, hyper_dev, scaler_state_dev, P.flags[rank], found_inf_dev, local_extras, L, C3,
+                       sync_state_dev);
 }

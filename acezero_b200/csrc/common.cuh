@@ -289,6 +289,10 @@ __host__ __device__ constexpr uint32_t make_idesc_f16(int m, int n, bool a_mn_ma
          ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 
+// GradScaler's overflow test of a weight gradient: autocast materialises weight gradients in fp16, so a value beyond the fp16
+// range (|g| > 65504) is an inf there even when the fp32 value is finite
+__device__ __forceinline__ bool fp16_grad_overflow(float g) { return !isfinite(g) || fabsf(g) > 65504.f; }
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

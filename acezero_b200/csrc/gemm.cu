@@ -228,13 +228,9 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         for (int j = 0; j < 8; ++j)
           dst[j] = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
                                __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
-        if (args.nonfinite != nullptr) {
-          // GradScaler check folded in: autocast materialises weight gradients in fp16, so |g| > 65504 is an overflow
+        if (args.nonfinite != nullptr) {  // GradScaler check folded in
 #pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const float g = __uint_as_float(v[j]);
-            bad |= !isfinite(g) || fabsf(g) > 65504.f;
-          }
+          for (int j = 0; j < 32; ++j) bad |= fp16_grad_overflow(__uint_as_float(v[j]));
         }
       }
     } else {
@@ -318,7 +314,7 @@ gemm_tcgen05_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       if (row_ok) {
         const float g = __uint_as_float(v[0]);
         args.bias_grad[(long long)z * args.bias_grad_zstride + row] = g;
-        bad |= !isfinite(g) || fabsf(g) > 65504.f;
+        bad |= fp16_grad_overflow(g);
       }
     }
     if (EPI != EPI_FWD && args.nonfinite != nullptr) {

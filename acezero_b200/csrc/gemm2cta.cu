@@ -272,13 +272,9 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
             reinterpret_cast<float4*>(dst)[j] = make_float4(__uint_as_float(v[4 * j]), __uint_as_float(v[4 * j + 1]),
                                                             __uint_as_float(v[4 * j + 2]), __uint_as_float(v[4 * j + 3]));
         }
-        if (args.nonfinite != nullptr) {
-          // GradScaler check folded in: autocast materialises weight gradients in fp16, so |g| > 65504 is an overflow
+        if (args.nonfinite != nullptr) {  // GradScaler check folded in
 #pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const float g = __uint_as_float(v[j]);
-            bad |= !isfinite(g) || fabsf(g) > 65504.f;
-          }
+          for (int j = 0; j < 32; ++j) bad |= fp16_grad_overflow(__uint_as_float(v[j]));
         }
       }
     if (bias_col && grp == 0) {
@@ -313,7 +309,7 @@ gemm2cta_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__
           const int grow = tm * 2 * T2_BM + rt;
           if (grow < args.M) {
             args.bias_grad[(long long)z * args.bias_grad_zstride + grow] = sum;
-            bad |= !isfinite(sum) || fabsf(sum) > 65504.f;
+            bad |= fp16_grad_overflow(sum);
           }
         }
         if (t128 == 0) args.bias_count[z * tiles_m + tm] = 0u;   // ready for the next launch

@@ -16,6 +16,7 @@
 
 #include <vector>
 
+#include "adamw.cuh"
 #include "gemm.cuh"
 #include "gemm2cta.cuh"
 #include "schedule.cuh"
@@ -23,9 +24,6 @@
 #include "repro_loss.cuh"
 
 namespace acez {
-
-static constexpr int kC = 512;  // head width, hard-coded in the reference (ace_network.py:76)
-static constexpr size_t kLayerStride = (size_t)kC * kC + kC;
 
 static inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
@@ -539,10 +537,10 @@ __global__ void fc3_reduce_kernel(const float* __restrict__ part, int nblk, int 
   bool bad = false;
   if (idx < total && sub == 0) {
     if (idx < 4 * kC) {
-      if (idx < C3 * kC) { gW3[idx] = s; bad = !isfinite(s) || fabsf(s) > 65504.f; }
+      if (idx < C3 * kC) { gW3[idx] = s; bad = fp16_grad_overflow(s); }
     } else if (idx - 4 * kC < C3) {
       gb3[idx - 4 * kC] = s;
-      bad = !isfinite(s) || fabsf(s) > 65504.f;
+      bad = fp16_grad_overflow(s);
     }
   }
   if (__syncthreads_or(bad ? 1 : 0) && threadIdx.x == 0 && nonfinite != nullptr) atomicOr(nonfinite, 1);
@@ -556,26 +554,9 @@ __global__ void grad_check_kernel(const float* __restrict__ g, size_t n, int* __
   pdl_wait();
   pdl_launch_dependents();
   bool bad = false;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-    const float v = g[i];
-    // under autocast the weight gradient is materialised in fp16: |g| > 65504 overflows to inf there
-    bad |= !isfinite(v) || fabsf(v) > 65504.f;
-  }
+  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x)
+    bad |= fp16_grad_overflow(g[i]);
   if (__syncthreads_or(bad ? 1 : 0) && threadIdx.x == 0) atomicOr(found_inf, 1);
-}
-
-__device__ __forceinline__ void scaler_update(float* st, int found, int use_scaler) {
-  // torch.cuda.amp.GradScaler.update(): backoff 0.5 on inf, growth x2 every 2000 clean steps
-  if (use_scaler && found) {
-    st[0] *= 0.5f;
-    st[1] = 0.f;
-  } else {
-    st[2] += 1.f;
-    if (use_scaler) {
-      st[1] += 1.f;
-      if (st[1] >= 2000.f) { st[0] *= 2.f; st[1] = 0.f; }
-    }
-  }
 }
 
 __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
@@ -586,21 +567,7 @@ __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
   pdl_launch_dependents();
   const int found = use_scaler ? *found_inf : 0;
   if (!found) {  // GradScaler.step skips optimizer.step() on inf/nan
-    const float lr = hyper[0], b1 = hyper[1], b2 = hyper[2], eps = hyper[3], wd = hyper[4];
-    const float inv_scale = use_scaler ? 1.f / scaler_state[0] : 1.f;
-    const float t = scaler_state[2] + 1.f;  // this step's index (torch: state['step'] += 1 before use)
-    const float bc1 = 1.f - powf(b1, t), bc2 = 1.f - powf(b2, t);
-    const float step_size = lr / bc1;
-    const float bc2_sqrt = sqrtf(bc2);
-    auto update = [&](float gi, float& pi, float& mi, float& vi) {
-      if (use_scaler) gi = __half2float(__float2half_rn(gi));  // fp16 weight gradient of the autocast conv
-      gi *= inv_scale;                                          // GradScaler.unscale_
-      pi *= (1.f - lr * wd);                                    // decoupled weight decay (torch adamw)
-      mi = mi + (1.f - b1) * (gi - mi);                         // exp_avg.lerp_(grad, 1 - beta1)
-      vi = b2 * vi + (1.f - b2) * gi * gi;
-      const float denom = sqrtf(vi) / bc2_sqrt + eps;
-      pi -= step_size * (mi / denom);
-    };
+    const AdamWStep adamw(hyper, scaler_state, use_scaler);
     const size_t n4 = n / 4;
     const size_t wsz = (size_t)kC * kC;
     const size_t tstride = (size_t)gridDim.x * blockDim.x;
@@ -621,10 +588,10 @@ __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
       if (q >= n4) continue;
       const float4 g4 = G[u];
       float4 p4 = P[u], m4 = M[u], v4 = V[u];
-      update(g4.x, p4.x, m4.x, v4.x);
-      update(g4.y, p4.y, m4.y, v4.y);
-      update(g4.z, p4.z, m4.z, v4.z);
-      update(g4.w, p4.w, m4.w, v4.w);
+      adamw.update(g4.x, p4.x, m4.x, v4.x);
+      adamw.update(g4.y, p4.y, m4.y, v4.y);
+      adamw.update(g4.z, p4.z, m4.z, v4.z);
+      adamw.update(g4.w, p4.w, m4.w, v4.w);
       reinterpret_cast<float4*>(p)[q] = p4;
       reinterpret_cast<float4*>(m)[q] = m4;
       reinterpret_cast<float4*>(v)[q] = v4;
@@ -646,7 +613,7 @@ __global__ void adamw_kernel(float* __restrict__ p, const float* __restrict__ g,
     }
     for (size_t i = 4 * n4 + (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
       float pi = p[i], mi = m[i], vi = v[i];
-      update(g[i], pi, mi, vi);
+      adamw.update(g[i], pi, mi, vi);
       p[i] = pi; m[i] = mi; v[i] = vi;
       if (W16 != nullptr) {
         const size_t l = i / kLayerStride, r = i % kLayerStride;
@@ -905,7 +872,7 @@ extern "C" size_t acez_head_param_count(const acez_head_config* cfg) {
   if (!cfg || cfg->num_res_blocks < 1) return 0;
   const int L = 3 * cfg->num_res_blocks + 2;
   const int C3 = cfg->use_homogeneous ? 4 : 3;
-  return (size_t)L * kLayerStride + (size_t)C3 * kC + C3;
+  return head_param_count(L, C3);
 }
 
 extern "C" size_t acez_head_workspace_bytes(const acez_head_config* cfg) {
