@@ -28,6 +28,7 @@ from ace_network import Regressor
 from acezero_b200 import _lib
 from acezero_b200 import posefile
 from acezero_b200.encoder import out_hw as encoder_out_hw
+from acezero_b200.imageprep import GpuImageDataset, ImagePrep
 from acezero_b200.parallel import rows_capacity_per_rank
 from acezero_b200.trainer import TrainLoop, BUFFER_KEYS
 
@@ -97,7 +98,14 @@ class TrainerACE:
                 aug_rotation=options.aug_rotation, aug_scale_max=options.aug_scale, aug_scale_min=1 / options.aug_scale,
                 image_short_size=options.image_resolution, use_half=options.use_half,
                 use_heuristic_focal_length=options.use_heuristic_focal_length)
+            if os.environ.get("ACEZ_GPU_IMAGES", "0") == "1" and not self.use_depth:
+                dataset = GpuImageDataset(dataset)
         self.dataset = dataset
+        # decode and random draws on the loader workers, pixel arithmetic in csrc/imageprep.cu (acezero_b200/imageprep.py)
+        self.gpu_images = isinstance(dataset, GpuImageDataset)
+        if self.gpu_images and (self.use_depth or not options.use_half):
+            raise NotImplementedError("the GPU image path prepares fp16 images without depth (use_half, no depth files "
+                                      "or pose seed)")
         if options.use_external_focal_length is not None:
             self.dataset.set_external_focal_length(options.use_external_focal_length)
         _logger.info("Loaded training scan from: {} -- {} images, mean: {:.2f} {:.2f} {:.2f}".format(
@@ -221,6 +229,10 @@ class TrainerACE:
         asynchronously from the loader's pinned tensors straight into the batch slot, the per-image matrices of a group
         travel as one pinned row block, an all-true mask costs no resize / copy, and one fused kernel per image scatters
         the sampled rows into all 8 buffer arrays. No host synchronisation per image.
+
+        With a GpuImageDataset the loader items carry raw uint8 pixels and the drawn augmentation parameters: the mask
+        cells are computed on the device for every image (every rank), and the owned images of a group are resized,
+        jittered, normalised and rotated by the csrc/imageprep.cu kernels straight into the batch slot.
         """
         o = self.options
         max_batch = max(1, int(os.environ.get("ACEZ_FILL_BATCH", "8") or 8))
@@ -243,6 +255,8 @@ class TrainerACE:
         # image of the loader order); single GPU: local == the final buffer
         local_cap = size if world == 1 else rows_capacity_per_rank(size, o.samples_per_image, world)
         d = self.device
+        gpu_images = self.gpu_images
+        prep = ImagePrep(d) if gpu_images else None
         buf = self._alloc_buffer(local_cap)
         lib = _lib.load()
         enc = self.regressor.encoder
@@ -268,8 +282,9 @@ class TrainerACE:
             if not group:
                 return
             n = len(group)
-            H_img, W_img = group[0]["image"].shape[2], group[0]["image"].shape[3]
-            images = torch.empty((n, 1, H_img, W_img), dtype=group[0]["image"].dtype, device=d)
+            H_img, W_img = group[0]["shape"][2], group[0]["shape"][3]
+            images = torch.empty((n, 1, H_img, W_img), dtype=torch.float16 if gpu_images else group[0]["image"].dtype,
+                                 device=d)
             sl = stage_next[0]
             stage_next[0] = (sl + 1) % n_stage
             if stage_events[sl] is not None:
@@ -277,10 +292,13 @@ class TrainerACE:
             else:
                 stage_events[sl] = torch.cuda.Event()
             for k, g in enumerate(group):
-                images[k].copy_(g["image"][0], non_blocking=True)             # pinned (loader) -> device, asynchronous
+                if not gpu_images:
+                    images[k].copy_(g["image"][0], non_blocking=True)         # pinned (loader) -> device, asynchronous
                 mats_np[sl][k] = g["mats"]
             mats_dev[sl][:n].copy_(mats_host[sl][:n], non_blocking=True)
             stage_events[sl].record()
+            if gpu_images:
+                prep.prepare([g["item"] for g in group], images)
             feats = enc.forward_nhwc(images)                                  # [n,h,w,512] fp16: ONE launch sequence
             _, H, W, C = feats.shape
             for k, g in enumerate(group):
@@ -299,21 +317,35 @@ class TrainerACE:
         with torch.no_grad():
             while buffer_idx < o.max_training_buffer_size and passes < o.max_dataset_passes:
                 passes += 1
-                for image, mask, pose_inv, aug_pose_inv, K, Kinv, crds, _, idx in loader:
-                    B = image.shape[0]
-                    assert B == 1, "the buffer is filled image by image (batch_size=1 sampler, reference :298-300)"
-                    H, W = encoder_out_hw(image.shape[2], image.shape[3])
-                    # mask at output resolution (reference :373-378), decided on the CPU copy: no GPU sync. An all-true mask
-                    # (no rotation augmentation) stays all-true under NEAREST resizing: no resize, no host->device copy
-                    if mask.numpy().all():
-                        if (H, W) not in ones_cache:
-                            ones_cache[(H, W)] = torch.ones(H * W, dtype=torch.float32, device=d)
-                        weights = ones_cache[(H, W)]
+                for item in loader:
+                    if gpu_images:
+                        image, crds, idx, B = None, None, item["idx"], 1
+                        shape = (1, 1) + tuple(item["size"])
+                        H, W = encoder_out_hw(shape[2], shape[3])
+                        if item["rotate"] and item["angle"] != 0.0:
+                            weights = prep.mask_cells(item, H, W)   # never empty (GpuImageDataset checks the size)
+                        else:
+                            if (H, W) not in ones_cache:
+                                ones_cache[(H, W)] = torch.ones(H * W, dtype=torch.float32, device=d)
+                            weights = ones_cache[(H, W)]
+                        mats = np.asarray(item["mats"], dtype=np.float32)
                     else:
-                        m = TF.resize(mask, [H, W], interpolation=TF.InterpolationMode.NEAREST).bool()
-                        if m.sum() == 0:
-                            continue
-                        weights = m.float().view(-1).to(d, non_blocking=True)
+                        image, mask, pose_inv, aug_pose_inv, K, Kinv, crds, _, idx = item
+                        shape = tuple(image.shape)
+                        B = image.shape[0]
+                        assert B == 1, "the buffer is filled image by image (batch_size=1 sampler, reference :298-300)"
+                        H, W = encoder_out_hw(image.shape[2], image.shape[3])
+                        # mask at output resolution (reference :373-378), decided on the CPU copy: no GPU sync. An all-true
+                        # mask (no rotation augmentation) stays all-true under NEAREST resizing: no resize, no host->device copy
+                        if mask.numpy().all():
+                            if (H, W) not in ones_cache:
+                                ones_cache[(H, W)] = torch.ones(H * W, dtype=torch.float32, device=d)
+                            weights = ones_cache[(H, W)]
+                        else:
+                            m = TF.resize(mask, [H, W], interpolation=TF.InterpolationMode.NEAREST).bool()
+                            if m.sum() == 0:
+                                continue
+                            weights = m.float().view(-1).to(d, non_blocking=True)
                     n_sel = min(o.samples_per_image * B, o.max_training_buffer_size - buffer_idx)
                     # EVERY rank draws the indices of EVERY image: the CUDA generator advances exactly as in a single-GPU run
                     sample_idxs = torch.multinomial(weights, n_sel, replacement=True,
@@ -323,12 +355,14 @@ class TrainerACE:
                     owner = image_counter % world
                     image_counter += 1
                     if owner == rank:
-                        if group and (group[0]["image"].shape != image.shape or len(group) == max_batch):
+                        if group and (group[0]["shape"] != shape or len(group) == max_batch):
                             flush()
-                        mats = np.concatenate([aug_pose_inv.numpy()[0, :3].ravel(), pose_inv.numpy()[0].ravel(),
-                                               K.numpy()[0].ravel(), Kinv.numpy()[0].ravel()]).astype(np.float32)
-                        group.append({"image": image, "mats": mats, "crds": crds, "idx": int(idx), "sample_idxs": sample_idxs,
-                                      "n_sel": n_sel, "local_row0": local_rows[rank], "hw": (H, W)})
+                        if not gpu_images:
+                            mats = np.concatenate([aug_pose_inv.numpy()[0, :3].ravel(), pose_inv.numpy()[0].ravel(),
+                                                   K.numpy()[0].ravel(), Kinv.numpy()[0].ravel()]).astype(np.float32)
+                        group.append({"image": image, "item": item if gpu_images else None, "shape": shape, "mats": mats,
+                                      "crds": crds, "idx": int(idx), "sample_idxs": sample_idxs, "n_sel": n_sel,
+                                      "local_row0": local_rows[rank], "hw": (H, W)})
                     records.append((owner, buffer_idx, n_sel, local_rows[owner]))
                     local_rows[owner] += n_sel
                     buffer_idx += n_sel

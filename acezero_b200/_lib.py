@@ -81,6 +81,15 @@ SCHED_STATE_FLOATS = 128
 SCHED_KINDS = {"constant": 0, "circle": 1, "1cyclepoly": 2}
 
 
+class ImagePrepDesc(C.Structure):
+    _fields_ = [
+        ("src", C.c_void_p), ("h_in", C.c_int), ("w_in", C.c_int), ("channels", C.c_int),
+        ("coef_x", C.c_void_p), ("coef_y", C.c_void_p), ("kx", C.c_int), ("ky", C.c_int),
+        ("contrast_first", C.c_int), ("brightness", C.c_float), ("contrast", C.c_float), ("rotate", C.c_int),
+        ("affine", C.c_double * 6),
+    ]
+
+
 class DsacDebug(C.Structure):
     _fields_ = [
         ("hyp_poses", C.c_void_p), ("hyp_scores", C.c_void_p), ("best", C.c_void_p), ("hyp_tries", C.c_void_p),
@@ -99,6 +108,7 @@ EXPORTS = [
     "acez_adamw_dp_shard", "acez_adamw_dp_step", "acez_head_w16_ptr", "acez_gather_rows", "acez_gather_rows_multi", "acez_buffer_fill", "acez_adamw_step", "acez_schedule_init", "acez_schedule_step", "acez_gather_rows_multi_sched", "acez_dsac_workspace_bytes", "acez_dsac_forward_rgb_batch",
     "acez_encoder_workspace_bytes", "acez_encoder_plan_create", "acez_encoder_plan_destroy", "acez_encoder_out_hw",
     "acez_encoder_forward", "acez_pointcloud_metrics",
+    "acez_image_prep_workspace_bytes", "acez_image_prep", "acez_image_mask_cells",
 ]
 
 
@@ -156,6 +166,16 @@ def load():
     lib.acez_encoder_out_hw.argtypes = [i, i, C.POINTER(i), C.POINTER(i)]
     lib.acez_encoder_forward.argtypes = [vp, vp, i, i, i, i, vp, vp]
     lib.acez_pointcloud_metrics.argtypes = [vp, i, i, i, vp, vp, i, vp, vp, vp, vp]
+    lib.acez_image_prep_workspace_bytes.argtypes = [C.POINTER(ImagePrepDesc), i, i, i]
+    lib.acez_image_prep_workspace_bytes.restype = C.c_size_t
+    lib.acez_image_prep.argtypes = [C.POINTER(ImagePrepDesc), i, i, i, vp, C.c_size_t, vp, vp]
+    lib.acez_image_mask_cells.argtypes = [C.POINTER(C.c_double), i, i, i, i, vp, vp]
+    lib.acez_host_resize_sample.argtypes = [vp, C.c_longlong, vp, i]
+    lib.acez_host_jitter.argtypes = [i, i, f, f, i]
+    lib.acez_host_normalize.restype = f
+    lib.acez_host_rotate_sample.argtypes = [C.POINTER(C.c_double), vp, i, i, i, i]
+    lib.acez_host_rotate_sample.restype = C.c_double
+    lib.acez_host_mask_cell.argtypes = [C.POINTER(C.c_double), i, i, i, i, i, i]
     _lib = lib
     return lib
 

@@ -166,3 +166,55 @@ class CachedDataset(Dataset):
         if isinstance(idx, list):
             return default_collate([self.items[i] for i in idx])
         return self.items[idx]
+
+
+def write_frames(out_dir, n_images, H=480, W=640, focal=525.0, seed=2089, ext="jpg", gray=(), device="cpu"):
+    """Render n BoxRoom frames to image files (`ext` "jpg" or "png"), tinted to RGB so that the three channels differ;
+    the frames whose index is in `gray` are written as single-channel PNGs. Returns (paths, camera-to-world poses)."""
+    from pathlib import Path
+    from PIL import Image
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    room = BoxRoom(seed, octave_shift=math.log2(max(float(focal), 1.0) / 262.5)).to(device)
+    poses = trajectory(n_images, seed)
+    tint = torch.tensor([1.0, 0.85, 0.6], device=device)
+    paths = []
+    for i, c2w in enumerate(poses):
+        img, _ = room.render(c2w, focal, H, W)
+        if i in gray:
+            path = out_dir / f"frame-{i:06d}.gray.png"
+            Image.fromarray((img * 255).round().byte().cpu().numpy(), mode="L").save(path)
+        else:
+            x = torch.stack([img * tint[0], img * tint[1] + 0.1 * (1 - img), img * tint[2] + 0.3 * img * img], -1)
+            path = out_dir / f"frame-{i:06d}.color.{ext}"
+            a = (x.clamp(0, 1) * 255).round().byte().cpu().numpy()
+            Image.fromarray(a, mode="RGB").save(path, **({"quality": 90} if ext == "jpg" else {}))
+        paths.append(str(path))
+    return paths, poses
+
+
+class FrameDataset(Dataset):
+    """A minimal file-backed CamLocDataset look-alike: the attributes the reference's `_get_single_item` reads
+    (augmentation settings, image files, poses, focal length). Items come from a wrapper (acezero_b200.imageprep
+    .GpuImageDataset or oracle.image_ref.ImageRefDataset), not from this class."""
+
+    def __init__(self, rgb_files, poses, focal=525.0, augment=True, aug_rotation=15, aug_scale_min=2 / 3,
+                 aug_scale_max=3 / 2, aug_black_white=0.1, image_short_size=480):
+        self.rgb_files = list(rgb_files)
+        self.poses = [p.clone() for p in poses]
+        self.focal = float(focal)
+        self.external_focal = None
+        self.augment, self.aug_rotation = augment, aug_rotation
+        self.aug_scale_min, self.aug_scale_max = aug_scale_min, aug_scale_max
+        self.aug_black_white, self.image_short_size = aug_black_white, image_short_size
+        self.valid_file_indices = np.arange(len(self.rgb_files))
+        self.mean_cam_center = torch.stack([p[:3, 3] for p in self.poses]).mean(0)
+
+    def __len__(self):
+        return len(self.rgb_files)
+
+    def set_external_focal_length(self, f):
+        self.external_focal = float(f)
+
+    def get_focal_length(self, idx):
+        return self.external_focal if self.external_focal is not None else self.focal

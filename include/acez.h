@@ -379,6 +379,33 @@ int acez_encoder_forward(acez_encoder_plan* plan, const void* image, int image_i
 int acez_pointcloud_metrics(const float* sc, int n, int h, int w, const float* pose_inv_n34, const float* K_n33,
                             int subsample, float* err, float* grad, float* depth, acez_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------------------------
+ * Augmented training images (reference dataset.py `_get_single_item` without depth, csrc/imageprep.cu): PIL bilinear
+ * resize of the decoded uint8 image, convert("L"), ColorJitter(brightness, contrast) through PIL ImageEnhance,
+ * ToTensor + Normalize(0.4, 0.25), scikit-image order-1 rotate (mode 'reflect', clip) and the fp16 store, bit for bit.
+ * All images of one call share the output size. Coefficient tables (acezero_b200/imageprep.py `resize_coeffs`) are
+ * int32 [out, 2 + k]: first source index, tap count, k Q22 weights.
+ * ---------------------------------------------------------------------------------------------------------- */
+typedef struct {
+  const uint8_t* src;        /* device [h_in, w_in, channels], channels 1 (gray) or 3 (RGB) */
+  int h_in, w_in, channels;
+  const int32_t* coef_x;     /* device [w_out, 2 + kx]; NULL exactly when w_in == w_out (PIL skips that pass) */
+  const int32_t* coef_y;     /* device [h_out, 2 + ky]; NULL exactly when h_in == h_out */
+  int kx, ky;
+  int contrast_first;        /* ColorJitter's randperm puts contrast before brightness */
+  float brightness, contrast;/* jitter factors; 1, 1 = no jitter */
+  int rotate;                /* 0: no rotation (augmentation off) */
+  double affine[6];          /* inverse map (col, row)_out -> (col, row)_in: the first two rows of skimage's matrix */
+} acez_image_prep_desc;
+
+size_t acez_image_prep_workspace_bytes(const acez_image_prep_desc* descs, int n, int h_out, int w_out);
+/* out: fp16 [n, 1, h_out, w_out] device. descs: host array. */
+int acez_image_prep(const acez_image_prep_desc* descs, int n, int h_out, int w_out, void* workspace,
+                    size_t workspace_bytes, void* out_f16, acez_stream_t stream);
+/* cells [h8*w8] float 0/1: the reference's rotated mask of an h x w image (affine6 as above, host memory) after
+ * TF.resize(mask, [h8, w8], NEAREST). */
+int acez_image_mask_cells(const double* affine6, int h, int w, int h8, int w8, float* cells, acez_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
